@@ -1,7 +1,7 @@
 """Contract benchmark: InterpGN training throughput on synthetic CHISCO-shaped EEG (BASELINE.json config 2:
 125 channels, T=1000, 3 classes, default shapelet set K=5 x L in {100,200,300,500}, FCN deep expert).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -15,6 +15,8 @@ of --batch samples (weak scaling).  Rank 0 prints ONE JSON line:
   cpu_baseline the CPU restatement of the reference path (oracle/, "port") timed on this box's host cores on a
                bounded sample (N=1 only)
 `--impl reference` times that CPU path alone under the same contract (rank 0 only).
+`--dump-outputs DIR` writes what the last timed step left (see last_step_arrays) as DIR/<name>.npy, so that two builds
+run with the same arguments, hence on the same seeded inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -23,6 +25,9 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "speech-imagery-eeg_b200"))
@@ -33,12 +38,13 @@ CONFIG2 = dict(enc_in=125, seq_len=1000, num_class=3)          # BASELINE.json c
 LENGTH_FRACS = [0.1, 0.2, 0.3, 0.5]
 K_PER_LEN = 5
 FP32_LANES_PER_SM = 128
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every mode of the workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=256, help="samples per GPU per step")
@@ -53,7 +59,14 @@ def parse():
     ap.add_argument("--no_extras", action="store_true", help="skip the cosine/3xtf32 mode, the same-GPU eager comparator "
                     "and the config-1 / config-5 lines (they run at N=1 only)")
     ap.add_argument("--amp", action="store_true", help="bf16 autocast for the deep expert (reference default is fp32 in its scripts)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss, model state and Adam moments after the last "
+                    "timed step as DIR/<name>.npy (rank 0; at most 64 MB in all, larger outputs as a seeded sample)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 def model_args(a):
@@ -254,6 +267,37 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
+def last_step_arrays(exp, loss):
+    """What a training step hands its caller, copied to the host: the loss and the model's state after the optimiser
+    step, plus Adam's moments, which carry that step's gradients (the step zeroes the gradients themselves)."""
+    out = {"loss": loss}
+    for k, v in exp.model.state_dict().items():
+        out["model." + k] = v
+    names = {p: n for n, p in exp.model.named_parameters()}
+    for p, st in exp.optimizer.state.items():
+        for k, v in st.items():
+            if k != "step":
+                out["adam.%s.%s" % (k, names[p])] = v
+    return {k: v.detach().cpu() for k, v in out.items()}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy, in float32 (float64 for float64 and integer tensors).  When they come
+    to more than DUMP_LIMIT_BYTES, each is cut to the same fraction of its elements, flattened, at positions drawn
+    from a generator seeded by its name: runs with the same arguments write the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrs = {k: v.to(torch.float32 if v.is_floating_point() and v.dtype != torch.float64 else torch.float64).numpy()
+            for k, v in arrays.items()}
+    budget = DUMP_LIMIT_BYTES - 1024 * len(arrs)        # 1 KiB a file for the .npy header
+    total = sum(a.nbytes for a in arrs.values())
+    for k, a in arrs.items():
+        if total > budget:
+            keep = max(1, a.size * budget // total)
+            idx = np.random.default_rng(zlib.crc32(k.encode())).choice(a.size, keep, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_ours(a, primary=True):
     """One measurement of this repo's training step under the contract: W warm-up, K timed steps with inputs resident
     (CUDA events, max over ranks), per-kernel rooflines from a second instrumented pass, and (primary only) the clock
@@ -310,10 +354,11 @@ def run_ours(a, primary=True):
     e0.record()
     for _ in range(a.steps):
         step_no += 1
-        exp.train_step(x, y, mask, 0, step_no)
+        loss = exp.train_step(x, y, mask, 0, step_no)
         marks.append(torch.cuda.Event(enable_timing=True)); marks[-1].record()
     e1.record()
     barrier()
+    last_step = last_step_arrays(exp, loss) if (primary and rank == 0 and a.dump_outputs) else None
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     if rank == 0:      # per-step spread of the timed region (diagnostic, stderr)
         prev, per = e0, []
@@ -384,6 +429,8 @@ def run_ours(a, primary=True):
     nbytes_allreduce = exp.grads.nbytes() if world > 1 else 0
     del exp
     torch.cuda.empty_cache()
+    if last_step is not None:
+        dump_outputs(a.dump_outputs, last_step)
     if rank != 0:
         return None
 
@@ -588,7 +635,7 @@ def main():
     if world == 1 and not a.no_extras:
         # the tensor-core engine in the same record: cosine distance, 3xTF32 operands (fp32-equivalent), same workload
         b = copy.copy(a)
-        b.distance_func, b.precision, b.steps = "cosine", "3xtf32", max(10, min(a.steps, 20))
+        b.distance_func, b.precision = "cosine", "3xtf32"
         m = run_ours(b, primary=False)
         line["modes"] = {"cosine_3xtf32": {k: m[k] for k in ("value", "unit", "ms_per_step", "steps", "warmup", "config",
                                                                "gpu_launches", "engines", "roofline", "rooflines",

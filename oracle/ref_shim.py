@@ -1,11 +1,11 @@
 """Import shim for the *live* reference modules (test infrastructure, NOT product code).
 
-Only usable in the authoring container, where /root/reference is mounted.  Nothing
-under tests/ -m gpu, smoke() or bench.py imports this file: it exists so that
-tests/golden/make_golden.py can run the unmodified reference
-(InterpretGatedNetwork/model/Shapelet.py, model/InterpGN.py) and freeze its outputs
+Only usable where IGN_REFERENCE_ROOT names a checkout of the reference
+(InterpretGatedNetwork); the repository does not carry it.  Nothing under tests/ -m gpu,
+smoke() or bench.py imports this file: it exists so that tests/golden/make_golden.py can
+run the unmodified reference (model/Shapelet.py, model/InterpGN.py) and freeze its outputs
 into tests/golden/*.npz, and so that `-m "not gpu"` tests can cross-check the oracle
-restatement against the real thing when the mount is present.
+restatement against the real thing when that checkout is given.
 
 The reference's directories are `model/` and `data_factory/` but its imports say
 `models.` / `data_provider.`; plotting dependencies are absent here.  We alias/stub
@@ -17,11 +17,11 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("IGN_REFERENCE_ROOT", "/root/reference/InterpretGatedNetwork")
+REF_ROOT = os.environ.get("IGN_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REF_ROOT, "model", "Shapelet.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_ROOT, "model", "Shapelet.py"))
 
 
 def _load(private_name, relpath):
@@ -40,7 +40,7 @@ def load_reference():
     if "ns" in _cache:
         return _cache["ns"]
     if not available():
-        raise RuntimeError("reference tree not mounted at %s" % REF_ROOT)
+        raise RuntimeError("no reference checkout at IGN_REFERENCE_ROOT=%r" % REF_ROOT)
     saved = {k: sys.modules.get(k) for k in (
         "utils", "utils.shapelet_util", "models", "models.Shapelet", "models.FullyConvNet",
         "models.PatchTST", "models.TimesNet", "models.Transformer", "models.ResNet",

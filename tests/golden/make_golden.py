@@ -1,12 +1,12 @@
-"""Generate golden vectors from the UNMODIFIED live reference (authoring container only).
+"""Generate golden vectors from the UNMODIFIED live reference.
 
-    python tests/golden/make_golden.py
+    IGN_REFERENCE_ROOT=<InterpretGatedNetwork checkout> python tests/golden/make_golden.py
 
-Imports /root/reference/InterpretGatedNetwork/model/{Shapelet,InterpGN,FullyConvNet}.py through
-oracle/ref_shim.py, runs them on seeded CPU inputs and freezes inputs + outputs + gradients into
-tests/golden/*.npz.  The reference has no tests/golden vectors of its own (SURVEY.md §4), so these
-files are the parity pin for oracle/ign_oracle.py and (through it, and directly) for the CUDA path.
-/root/reference does not travel to the GPU box; the .npz files do.
+Imports the reference's model/{Shapelet,InterpGN,FullyConvNet}.py through oracle/ref_shim.py, runs them
+on seeded CPU inputs and freezes inputs + outputs + gradients into tests/golden/*.npz.  The reference
+has no tests/golden vectors of its own (SURVEY.md §4), so these files are the parity pin for
+oracle/ign_oracle.py and (through it, and directly) for the CUDA path.  The repository does not carry
+the reference; the .npz files are what the tests compare against.
 """
 import os
 import sys

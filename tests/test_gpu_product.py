@@ -192,15 +192,19 @@ def test_cuda_graph_replay_is_the_same_training_as_the_eager_step(tmp_path, monk
         assert abs(le - lg) <= 1e-4 * abs(le) + 1e-6, (params["eager"][1], params["graph"][1])
 
 
-def test_bench_line_contract_of_our_arm():
+def test_bench_line_contract_of_our_arm(tmp_path):
     """`python bench.py` on one GPU (small batch, few steps, no extras): ONE JSON line with every key the measurement
     contract names — whole-job value, end-to-end object with its copy sizes, launch count, clocks, a roofline for the
-    dominant kernel with live timing, per-kernel entries, engines as the library reported them."""
+    dominant kernel with live timing, per-kernel entries, engines as the library reported them — and the last timed
+    step's outputs as .npy files."""
     import json
+    import numpy as np
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     env = {k: v for k, v in os.environ.items() if k not in ("RANK", "WORLD_SIZE", "LOCAL_RANK")}
+    dump = tmp_path / "outputs"
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "3", "--warmup", "3", "--batch", "16",
-                          "--no_extras", "--no_cpu_baseline"], capture_output=True, text=True, env=env, timeout=600)
+                          "--no_extras", "--no_cpu_baseline", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, env=env, timeout=600)
     assert out.returncode == 0, out.stderr[-3000:]
     lines = [ln for ln in out.stdout.strip().splitlines() if ln.startswith("{")]
     assert len(lines) == 1
@@ -221,3 +225,9 @@ def test_bench_line_contract_of_our_arm():
     names = {k["kernel"] for k in d["rooflines"]}
     assert {"shapelet_fwd", "shapelet_bwd", "bwd.pool_bwd", "bwd.tie_check", "bwd.contraction", "instnorm"} <= names
     assert set(d["engines"].values()) == {"fp32"}               # the default L1 distance has no tensor-core form
+    files = {p.name: np.load(p) for p in dump.iterdir()}
+    assert files["loss.npy"].shape == () and np.isfinite(files["loss.npy"])
+    assert files["model.sbm.shapelets.0.weights.npy"].shape == (5, 125, 100)
+    assert files["adam.exp_avg.sbm.shapelets.3.weights.npy"].shape == (5, 125, 500)
+    assert all(v.dtype in (np.float32, np.float64) and np.isfinite(v).all() for v in files.values())
+    assert sum(p.stat().st_size for p in dump.iterdir()) <= 64 * 10 ** 6

@@ -122,6 +122,28 @@ def test_transformer_expert_matches_reference_golden_on_cpu():
     assert torch.allclose(out, torch.as_tensor(g["dnn_preds"]), rtol=1e-4, atol=1e-5)
 
 
+def test_bench_dump_outputs_keeps_its_size_limit_and_samples_the_same_positions_every_run(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 .npy files; past the size limit, a sample at positions fixed by name."""
+    import os
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(0)
+    arrays = {"loss": torch.tensor(1.5), "model.w": torch.randn(300, 40, generator=g), "model.n": torch.tensor(7),
+              "model.h": torch.randn(1000, generator=g).half()}
+    bench.dump_outputs(str(tmp_path / "full"), arrays)
+    full = {k: np.load(tmp_path / "full" / (k + ".npy")) for k in arrays}
+    assert [full[k].dtype for k in arrays] == [np.float32, np.float32, np.float64, np.float32]
+    assert np.array_equal(full["model.w"], arrays["model.w"].numpy()) and float(full["model.n"]) == 7.0
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4 * 1024 + 20000)        # 20000 payload bytes for 52012
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    assert sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir()) <= bench.DUMP_LIMIT_BYTES
+    for k in arrays:
+        a, b = np.load(tmp_path / "a" / (k + ".npy")), np.load(tmp_path / "b" / (k + ".npy"))
+        assert np.array_equal(a, b) and np.isin(a, full[k]).all()
+    assert 0 < np.load(tmp_path / "a" / "model.w.npy").size < 300 * 40
+
+
 def test_reference_arm_line_contract():
     """`bench.py --impl reference` (the oracle port timed on the host cores): one JSON line with the bench contract's keys
     on rank 0, silence and exit 0 on the other ranks of a torchrun launch."""

@@ -34,7 +34,7 @@ def test_expert_restatement_matches_reference_golden(name):
 def test_expert_restatement_against_live_reference_if_mounted():
     import ref_shim
     if not ref_shim.available():
-        pytest.skip("reference tree not mounted")
+        pytest.skip("IGN_REFERENCE_ROOT does not name a reference checkout")
     ns = ref_shim.load_reference()
     torch.manual_seed(3)
     cfg = SimpleNamespace(enc_in=5, num_class=4, seq_len=40, dropout=0.0, activation="gelu", d_model=16, n_heads=2,
