@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define IGN_ABI_VERSION 2
+#define IGN_ABI_VERSION 3
 
 typedef enum {
   IGN_OK = 0,
@@ -101,22 +101,10 @@ int32_t ign_padded_windows(int32_t T, int32_t L, int32_t stride);
 int32_t ign_instnorm_forward(const float* x_dev, float* xn_dev, float* mean_dev, float* rstd_dev,
                              int32_t B, int32_t T, int32_t M, void* stream);
 
-/* pitch (doubles) of one prefix-sum row: T+4 rounded up to a multiple of 4 (32-byte rows) */
-int32_t ign_prefix_pitch(int32_t T);
-
-/* Sliding-window statistics for the norm terms of cosine / pearson / sql2 (fp64 exclusive prefix sums):
- *   P1[b,m,j] = sum_{i<j} xn[b,m,i], P2[b,m,j] = sum_{i<j} xn[b,m,i]^2, j in [0,T].
- *   Storage: row pitch ign_prefix_pitch(T); P[j] is at slot 3+j of its row (slots 0..2 are zero padding, so
- *   the kernel's 4-sample runs are 32-byte aligned).  ||x_w||^2 of the window starting at sample j0 is
- *   P2[j0+L]-P2[j0]; its sum is P1[j0+L]-P1[j0].  (Stand-alone form of the pass; the distance kernels consume
- *   the fused per-group output of ign_window_stats below.) */
-int32_t ign_window_prefix(const float* xn_dev, double* pre1_dev, double* pre2_dev,
-                          int32_t B, int32_t M, int32_t T, void* stream);
-
 /* pitch (floats) of one window-statistics row: T' rounded up to a multiple of 16 */
 int32_t ign_stats_pitch(int32_t T, int32_t L, int32_t stride);
 
-/* The sliding-window prefix-sum pass in the form the distance kernels consume: for G (<= 8) length groups at
+/* Sliding-window statistics for the norm terms of cosine / pearson / sql2: for G (<= 8) length groups at
  * once, per series row an fp64 prefix scan of xn and xn^2 in shared memory, then per window the fp32 norm term
  *   SQL2: st0 = ||x_w||^2      COSINE: st0 = 1/max(||x_w||,1e-8)      PEARSON: st0 = ||x_w-mu||, st1 = mu
  * The pad slots t >= T' of st0 hold an ignore marker (+inf for SQL2, NaN for COSINE / PEARSON: the resulting
@@ -179,30 +167,20 @@ size_t ign_shapelet_backward_recompute_workspace(const ign_shapelet_desc* desc, 
    then the threshold of lts_min is needed again: threshold_dev below, NULL otherwise allowed).
  *   dmin_dev / argmin_dev [B,K,M]: the forward's outputs; required for lts_min (its hard index and soft-min
  *   shift), ignored (may be NULL) for rbf_max, whose arg-max-of-p one-hot is re-derived from dstore.
- *   dW_dev [K,M,L] is overwritten (not accumulated).  Deterministic (no float atomics). */
+ *   dW_dev [K,M,L] is overwritten (not accumulated).  Deterministic (no float atomics).
+ *   dW_dev == NULL (weights frozen, only the input gradient wanted): runs the preparation alone — the pooling backward
+ *   and, for PEARSON, the shapelet norms — which leaves in the workspace the coefficients ign_shapelet_backward_input
+ *   reads; the contraction is skipped.  Stored-distance mode only (dstore_dev != NULL). */
 int32_t ign_shapelet_backward(const ign_shapelet_desc* desc, const float* xn_dev, const float* st0_dev,
                               const float* st1_dev, const float* W_dev, const float* threshold_dev,
                               const float* g_dev, const float* dstore_dev, const float* dmin_dev,
                               const int32_t* argmin_dev, float* dW_dev, void* workspace_dev,
                               size_t workspace_bytes, void* stream);
 
-/* The same call split in two, for callers that own several length groups (ShapeBottleneckModel has four): the
- * PREPARE phase (pooling backward, L1 tie pre-check: HBM / L2-bound, a few hundred microseconds) of the next groups
- * can be issued on a second stream under the compute-bound CONTRACT phase (contraction + finalize -> dW) of the current
- * one.  Both phases take the same arguments and the same workspace; CONTRACT must be ordered after PREPARE of its own
- * group (stream order or an event).  Stored-distance mode only (dstore_dev != NULL). */
-#define IGN_BWD_PREPARE 1
-#define IGN_BWD_CONTRACT 2
-int32_t ign_shapelet_backward_phases(const ign_shapelet_desc* desc, const float* xn_dev, const float* st0_dev,
-                                     const float* st1_dev, const float* W_dev, const float* threshold_dev,
-                                     const float* g_dev, const float* dstore_dev, const float* dmin_dev,
-                                     const int32_t* argmin_dev, float* dW_dev, void* workspace_dev,
-                                     size_t workspace_bytes, int32_t phases, void* stream);
-
 /* Gradient w.r.t. the normalised input series — what autograd gives a user of the reference who asks for input
  * gradients (saliency, gradcheck) through Shapelet.forward; the training loop never does
- * (experiment_classification.py:315).  Call AFTER ign_shapelet_backward (or its PREPARE phase) of the same group with
- * the same workspace: it reads the per-window coefficients that call left there.
+ * (experiment_classification.py:315).  Call AFTER ign_shapelet_backward (with or without dW_dev) of the same group
+ * with the same workspace: it reads the per-window coefficients that call left there.
  *   dxn_dev [B,M,Tp] += sum_k sum_t dLoss/dd[b,k,t] * d d_t / d xn[b,m,t*stride + l]     (ADDED: zero it once, call per group)
  * L1 (Shapelet.py:74, sign(0) = 0), cosine (:64-66), pearson (:11-19,:67-69).  SQL2: nothing is added — the
  * reference's ShapeletDistanceFunc.backward returns zeros for its input (Shapelet.py:40).  Stored-distance mode only. */

@@ -111,19 +111,12 @@ int32_t ign_debug_tc_profile(uint64_t* host16, int32_t reset) {
 int32_t ign_padded_len(int32_t T) { return padded_len(T); }
 int32_t ign_num_windows(int32_t T, int32_t L, int32_t stride) { return (L <= 0 || stride <= 0) ? 0 : num_windows(T, L, stride); }
 int32_t ign_padded_windows(int32_t T, int32_t L, int32_t stride) { return (L <= 0 || stride <= 0) ? 0 : padded_windows(T, L, stride); }
-int32_t ign_prefix_pitch(int32_t T) { return prefix_pitch(T); }
 
 int32_t ign_instnorm_forward(const float* x, float* xn, float* mean, float* rstd, int32_t B, int32_t T,
                              int32_t M, void* stream) {
   IGN_REQUIRE(x && xn, "instnorm_forward: null pointer");
   IGN_REQUIRE(B > 0 && T > 0 && M > 0 && B <= 65535, "instnorm_forward: bad shape B=%d T=%d M=%d", B, T, M);
   return launch_instnorm(x, xn, mean, rstd, B, T, M, (cudaStream_t)stream);
-}
-
-int32_t ign_window_prefix(const float* xn, double* pre1, double* pre2, int32_t B, int32_t M, int32_t T, void* stream) {
-  IGN_REQUIRE(xn && pre1 && pre2, "window_prefix: null pointer");
-  IGN_REQUIRE(B > 0 && T > 0 && M > 0, "window_prefix: bad shape B=%d T=%d M=%d", B, T, M);
-  return launch_prefix(xn, pre1, pre2, B, M, T, (cudaStream_t)stream);
 }
 
 int32_t ign_stats_pitch(int32_t T, int32_t L, int32_t stride) { return (L <= 0 || stride <= 0) ? 0 : stats_pitch(T, L, stride); }
@@ -189,27 +182,18 @@ int32_t ign_shapelet_backward(const ign_shapelet_desc* d, const float* xn, const
                               const float* W, const float* thr, const float* g, const float* dstore,
                               const float* dmin, const int32_t* argmin, float* dW, void* ws, size_t ws_bytes,
                               void* stream) {
-  return ign_shapelet_backward_phases(d, xn, st0, st1, W, thr, g, dstore, dmin, argmin, dW, ws, ws_bytes,
-                                      IGN_BWD_PREPARE | IGN_BWD_CONTRACT, stream);
-}
-
-int32_t ign_shapelet_backward_phases(const ign_shapelet_desc* d, const float* xn, const float* st0, const float* st1,
-                                     const float* W, const float* thr, const float* g, const float* dstore,
-                                     const float* dmin, const int32_t* argmin, float* dW, void* ws, size_t ws_bytes,
-                                     int32_t phases, void* stream) {
   int rc = check_desc(d, "shapelet_backward");
   if (rc) return rc;
-  IGN_REQUIRE(xn && W && g && dW && ws, "shapelet_backward: null pointer");
+  IGN_REQUIRE(xn && W && g && ws, "shapelet_backward: null pointer");
   IGN_REQUIRE(d->dist == IGN_DIST_L1 || st0, "shapelet_backward: dist %d needs the window statistics", d->dist);
   IGN_REQUIRE(d->dist != IGN_DIST_PEARSON || st1, "shapelet_backward: PEARSON needs st1 (window means)");
-  IGN_REQUIRE(phases >= 1 && phases <= 3, "shapelet_backward: phases must be IGN_BWD_PREPARE, IGN_BWD_CONTRACT or both");
   if (!dstore) {   // recompute mode: nothing was kept by the forward
-    IGN_REQUIRE(phases == 3, "shapelet_backward(recompute): the phases cannot be split (the workspace is reused per chunk)");
+    IGN_REQUIRE(dW, "shapelet_backward(recompute): dW is required (dW == NULL needs the stored distances)");
     IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || thr, "shapelet_backward(recompute): lts_min needs the threshold again");
     return launch_shapelet_bwd_recompute(*d, xn, st0, st1, W, thr, g, dW, ws, ws_bytes, (cudaStream_t)stream);
   }
   IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || (dmin && argmin), "shapelet_backward: lts_min needs the forward's dmin and argmin");
-  return launch_shapelet_bwd_simt(*d, xn, st0, st1, W, g, d->K, 0, dstore, dmin, argmin, dW, ws, ws_bytes, phases,
+  return launch_shapelet_bwd_simt(*d, xn, st0, st1, W, g, d->K, 0, dstore, dmin, argmin, dW, ws, ws_bytes,
                                   (cudaStream_t)stream);
 }
 

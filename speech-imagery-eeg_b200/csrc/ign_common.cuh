@@ -35,9 +35,6 @@ __host__ __device__ inline int ceil_div(int a, int b) { return (a + b - 1) / b; 
 inline int padded_len(int T) { return round_up(T, 4); }
 inline int num_windows(int T, int L, int s) { return T < L ? 0 : (T - L) / s + 1; }
 inline int padded_windows(int T, int L, int s) { return round_up(num_windows(T, L, s), 4); }
-// fp64 prefix rows: pitch (doubles) and the slot of P[0]; P[j] lives at row*pitch + kPrefixOrigin + j
-constexpr int kPrefixOrigin = 3;
-__host__ __device__ inline int prefix_pitch(int T) { return round_up(T + 4, 4); }
 // per-group fp32 window statistics: row pitch = windows rounded up to 16 (zero padded)
 inline int stats_pitch(int T, int L, int s) { return round_up(num_windows(T, L, s), 16); }
 constexpr int kMaxStatGroups = 8;
@@ -46,18 +43,18 @@ struct StatGroups { int n; int L[kMaxStatGroups], s[kMaxStatGroups], Tw[kMaxStat
 // ---- launchers implemented in the .cu files (all asynchronous on `st`) ----
 int launch_instnorm(const float* x, float* xn, float* mean, float* rstd, int B, int T, int M,
                     cudaStream_t st);
-int launch_prefix(const float* xn, double* pre1, double* pre2, int B, int M, int T, cudaStream_t st);
 int launch_window_stats(const float* xn, const StatGroups& G, int B, int M, int T, int dist, cudaStream_t st);
 int launch_shapelet_fwd_simt(const ign_shapelet_desc& d, const float* xn, const float* st0,
                              const float* W, const float* thr, float* p, float* dmin,
                              int* argmin, float* dstore, cudaStream_t st);
 size_t shapelet_bwd_workspace_simt(const ign_shapelet_desc& d);
 // g [B,gK,M]: the launch's K shapelets are gk0 .. gk0+K-1 of it; dstore == NULL: the distances sit in the coefficient
-// buffer of the workspace already (recompute mode) and are converted in place
+// buffer of the workspace already (recompute mode) and are converted in place; dW == NULL: the preparation alone (the
+// coefficients for launch_shapelet_dx), no contraction
 int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const float* st0,
                              const float* st1, const float* W, const float* g, int gK, int gk0, const float* dstore,
                              const float* dmin, const int* argmin, float* dW, void* ws, size_t ws_bytes,
-                             int phases, cudaStream_t st);
+                             cudaStream_t st);
 bool shapelet_bwd_coef_offset(const ign_shapelet_desc& d, size_t* off_floats, size_t* total_bytes);
 int launch_shapelet_dx(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1, const float* W,
                        const float* coef, const float* dstore, float* dxn, cudaStream_t st);

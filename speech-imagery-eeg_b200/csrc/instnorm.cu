@@ -2,9 +2,9 @@
 //
 //   instnorm_kernel : x[B,T,M] (channels last) -> xn[B,M,Tp] (time contiguous, 16-byte rows)
 //                     reference: Shapelet.py:186-187  (x-mean_T)/(std_T(unbiased)+1e-8)
-//   prefix_kernel   : fp64 exclusive prefix sums of xn and xn^2 per series, from which every window's
-//                     sum / squared norm is one subtraction (norm terms of cosine/pearson/sql2,
-//                     Shapelet.py:11-19,28,64-66)
+//   window_stats_kernel : fp64 prefix sums of xn and xn^2 per series, from which every window's sum / squared
+//                     norm is one subtraction, turned into the norm terms of cosine/pearson/sql2
+//                     (Shapelet.py:11-19,28,64-66) for several length groups at once
 #include "ign_common.cuh"
 
 #include <cooperative_groups.h>
@@ -272,50 +272,6 @@ __device__ __forceinline__ double warp_incl_scan(double v, int lane) {
   return v;
 }
 
-// One warp per series row; each lane owns 4 consecutive samples per 128-sample chunk.  Row layout (pitch PP
-// doubles, 32-byte aligned): [3] = P[0] = 0, [4+j] = P[j+1], so each lane's four results form one aligned
-// 32-byte run and are written with two 16-byte stores.
-__global__ void __launch_bounds__(256) prefix_kernel(const float* __restrict__ xn,
-                                                     double* __restrict__ pre1,
-                                                     double* __restrict__ pre2, int rows, int T, int Tp,
-                                                     int PP) {
-  const int lane = threadIdx.x & 31;
-  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (row >= rows) return;
-  const float* xr = xn + (size_t)row * Tp;
-  double* o1 = pre1 + (size_t)row * PP;
-  double* o2 = pre2 + (size_t)row * PP;
-  double c1 = 0.0, c2 = 0.0;
-  if (lane < 4) { o1[lane] = 0.0; o2[lane] = 0.0; }
-  const int nchunk = (T + 127) / 128;
-  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (lane * 4 < Tp) v = *reinterpret_cast<const float4*>(xr + lane * 4);
-  for (int ch = 0; ch < nchunk; ++ch) {
-    const int j = ch * 128 + lane * 4;
-    float4 nv = make_float4(0.f, 0.f, 0.f, 0.f);           // prefetch the next chunk before the scan
-    if (ch + 1 < nchunk && j + 128 < Tp) nv = *reinterpret_cast<const float4*>(xr + j + 128);
-    double a0 = v.x, a1 = a0 + (double)v.y, a2 = a1 + (double)v.z, a3 = a2 + (double)v.w;
-    double q0 = (double)v.x * v.x, q1 = q0 + (double)v.y * v.y, q2 = q1 + (double)v.z * v.z,
-           q3 = q2 + (double)v.w * v.w;
-    const double s1 = warp_incl_scan(a3, lane), s2 = warp_incl_scan(q3, lane);
-    const double e1 = c1 + s1 - a3, e2 = c2 + s2 - q3;     // exclusive offset of this lane
-    if (j + 3 < T) {                                        // whole 32-byte run in range (pad slots absorb the tail)
-      *reinterpret_cast<double2*>(o1 + 4 + j) = make_double2(e1 + a0, e1 + a1);
-      *reinterpret_cast<double2*>(o1 + 6 + j) = make_double2(e1 + a2, e1 + a3);
-      *reinterpret_cast<double2*>(o2 + 4 + j) = make_double2(e2 + q0, e2 + q1);
-      *reinterpret_cast<double2*>(o2 + 6 + j) = make_double2(e2 + q2, e2 + q3);
-    } else {
-      if (j + 0 < T) { o1[4 + j] = e1 + a0; o2[4 + j] = e2 + q0; }
-      if (j + 1 < T) { o1[5 + j] = e1 + a1; o2[5 + j] = e2 + q1; }
-      if (j + 2 < T) { o1[6 + j] = e1 + a2; o2[6 + j] = e2 + q2; }
-    }
-    c1 += __shfl_sync(0xffffffffu, s1, 31);
-    c2 += __shfl_sync(0xffffffffu, s2, 31);
-    v = nv;
-  }
-}
-
-
 // Sliding-window statistics for all length groups in one pass: per series row an fp64 prefix scan of x and
 // x^2 in shared memory, then for every group g and window t the norm term its distance needs, as fp32:
 //   sql2    st0 = ||x_w||^2            cosine  st0 = 1/max(||x_w||,1e-8)
@@ -550,13 +506,6 @@ int launch_instnorm(const float* x, float* xn, float* mean, float* rstd, int B, 
     dim3 grid(ceil_div(M, 32), B);
     instnorm_kernel<<<grid, kNormThreads, 0, st>>>(x, xn, mean, rstd, T, M, Tp);
   }
-  IGN_CUDA(cudaGetLastError());
-  return IGN_OK;
-}
-
-int launch_prefix(const float* xn, double* pre1, double* pre2, int B, int M, int T, cudaStream_t st) {
-  const int rows = B * M;
-  prefix_kernel<<<ceil_div(rows, 8), 256, 0, st>>>(xn, pre1, pre2, rows, T, padded_len(T), prefix_pitch(T));
   IGN_CUDA(cudaGetLastError());
   return IGN_OK;
 }

@@ -1574,11 +1574,7 @@ size_t shapelet_bwd_workspace_simt(const ign_shapelet_desc& d) {
 int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const float* st0,
                              const float* st1, const float* W, const float* gr, int gK, int gk0, const float* dstore,
                              const float* dmin, const int* argmin, float* dW, void* ws, size_t ws_bytes,
-                             int phases, cudaStream_t st) {
-  // phases: bit 0 = preparation (pooling backward, pearson shapelet norms, L1 tie pre-check: HBM / L2-bound, needs
-  // only the forward's saved tensors and g), bit 1 = contraction + finalize (compute-bound).  A caller that owns
-  // several length groups issues the preparation of the next groups on a second stream under the contraction of the
-  // current one (layers/shapelet_ops.py).
+                             cudaStream_t st) {
   Geo g; BwdPlan bp;
   if (!base_geo(d, g)) { set_error("shapelet_backward: T=%d < L=%d", d.T, d.L); return IGN_ERR_INVALID; }
   if (!plan_bwd(g, bp)) { set_error("shapelet_backward: problem does not fit shared memory (T=%d L=%d)", d.T, d.L); return IGN_ERR_UNSUPPORTED; }
@@ -1588,9 +1584,8 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
   if (((uintptr_t)ws & 15) != 0) { set_error("shapelet_backward: workspace must be 16-byte aligned"); return IGN_ERR_INVALID; }
   float* base = reinterpret_cast<float*>(ws);
   const bool use_tc = shapelet_bwd_tc_supported(d);
-  const bool use_tie = !use_tc && d.dist == IGN_DIST_L1 && bp.hcap;
+  const bool use_tie = dW && !use_tc && d.dist == IGN_DIST_L1 && bp.hcap;   // the tie flags serve the contraction only
   unsigned char* tflags = reinterpret_cast<unsigned char*>(base + wo.tie);
-  if (phases & 1) {
   // 1. pooling backward (elementwise, HBM-bound): d -> per-window coefficients + per-row scalars
   if (d.dist == IGN_DIST_PEARSON) {
     shapelet_centred_norm_kernel<<<ceil_div(d.K * d.M, 8), 256, 0, st>>>(W, base + wo.wstat, d.K * d.M, d.L);
@@ -1655,8 +1650,7 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
                                                                g.nkb, bp.hcap, bsplit);
     IGN_CUDA(cudaGetLastError());
   }
-  }   // phases & 1
-  if (!(phases & 2)) return IGN_OK;
+  if (!dW) return IGN_OK;     // input gradient only: the coefficients are what launch_shapelet_dx reads
   // 2. contraction with the series into per-chunk partials: tensor pipe for the cross-term modes in the tcgen05
   //    precisions (shapelet_tc_bwd.cu), FP32 pipe otherwise
   if (use_tc) {
@@ -1752,7 +1746,7 @@ int launch_shapelet_bwd_recompute(const ign_shapelet_desc& d, const float* xn, c
     if (rc1) return rc1;
     // 2. pooling backward in place, contraction, finalize -> dW[k0 .. k0+Kc)
     rc1 = launch_shapelet_bwd_simt(dc, xn, st0, st1, W + wofs, gr, d.K, k0, nullptr, outp + no,
-                                   reinterpret_cast<const int*>(outp + 2 * no), dW + wofs, ws, rc.bwd_bytes, 3, st);
+                                   reinterpret_cast<const int*>(outp + 2 * no), dW + wofs, ws, rc.bwd_bytes, st);
     if (rc1) return rc1;
   }
   return IGN_OK;

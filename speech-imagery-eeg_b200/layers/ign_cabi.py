@@ -10,12 +10,11 @@ from ctypes import POINTER, Structure, c_char_p, c_double, c_float, c_int32, c_s
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("IGN_B200_LIB", os.path.join(_HERE, "..", "lib", "libign_b200.so"))
 
-IGN_ABI_VERSION = 2
+IGN_ABI_VERSION = 3
 DIST = {"l1": 0, "sql2": 1, "cosine": 2, "pearson": 3}
 POOL = {"rbf_max": 0, "lts_min": 1}
 PRECISION = {"fp32": 0, "3xtf32": 1, "tf32": 2}
 ENGINE = {0: "fp32", 1: "tcgen05"}
-BWD_PREPARE, BWD_CONTRACT = 1, 2
 
 
 class ShapeletDesc(Structure):
@@ -43,9 +42,7 @@ _SIGNATURES = {
     "ign_padded_len": (c_int32, [c_int32]),
     "ign_num_windows": (c_int32, [c_int32, c_int32, c_int32]),
     "ign_padded_windows": (c_int32, [c_int32, c_int32, c_int32]),
-    "ign_prefix_pitch": (c_int32, [c_int32]),
     "ign_instnorm_forward": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, _P]),
-    "ign_window_prefix": (c_int32, [_P, _P, _P, c_int32, c_int32, c_int32, _P]),
     "ign_stats_pitch": (c_int32, [c_int32, c_int32, c_int32]),
     "ign_window_stats": (c_int32, [_P, c_int32, c_int32, c_int32, c_int32, POINTER(c_int32), POINTER(c_int32), c_int32,
                                    POINTER(_P), POINTER(_P), _P]),
@@ -56,7 +53,6 @@ _SIGNATURES = {
     "ign_shapelet_dstore_bytes": (c_size_t, [POINTER(ShapeletDesc)]),
     "ign_shapelet_backward_recompute_workspace": (c_size_t, [POINTER(ShapeletDesc), c_size_t]),
     "ign_shapelet_backward": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 11 + [c_size_t, _P]),
-    "ign_shapelet_backward_phases": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 11 + [c_size_t, c_int32, _P]),
     "ign_shapelet_backward_input": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 7 + [c_size_t, _P]),
     "ign_diversity_partials": (c_int32, [c_int32]),
     "ign_diversity_forward": (c_int32, [_P, _P, _P, c_int32, c_int32, c_int32, _P]),

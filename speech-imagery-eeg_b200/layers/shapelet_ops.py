@@ -10,7 +10,7 @@ from __future__ import annotations
 
 import os
 from ctypes import byref, c_int32, c_void_p
-from typing import Optional, Tuple
+from typing import Optional
 
 import torch
 
@@ -22,8 +22,9 @@ _DIST_OF_FLAG = {"cosine": "cosine", "pearson": "pearson"}
 # coefficient workspace of the same size (stored-distance mode: fastest, 2 x 4*B*M*K*T' bytes).  Above it the layer
 # switches to the recompute backward (nothing saved, shapelets walked in chunks inside a workspace of at most this
 # size): config 2 at B=256 needs 1.2 GB per group and stores, so do the K = 100 points of the config-4 sweep (23 GB);
-# the K = 1000 points would need 232 GB and recompute.  Four groups at the limit keep 4 x 16 GiB of distances plus one
-# 16 GiB coefficient buffer: under 80 GiB of the 180.
+# the K = 1000 points would need 232 GB and recompute.  The saved distances of every stored group are live from the
+# forward until the backward; the backward allocates one group's workspace at a time and releases it before the next
+# group's.  Four groups at the limit keep 4 x 16 GiB of distances plus one 16 GiB workspace: under 80 GiB of the 180.
 STORE_BUDGET_BYTES = int(float(os.environ.get("IGN_BWD_STORE_BUDGET_GB", "32")) * 2 ** 30)
 
 
@@ -105,13 +106,12 @@ def _check_device(dev: torch.device):
 
 class SeriesPack:
     """Instance-normalised series in the kernels' layout: xn [B,M,Tp] fp32 (time contiguous, zero padded
-    to a multiple of 4) plus lazily built fp64 window prefix sums shared by all length groups."""
+    to a multiple of 4) plus the lazily built window statistics of each length group."""
 
     def __init__(self, xn: torch.Tensor, T: int, xn_var: Optional[torch.Tensor] = None):
         self.xn = xn               # the kernels' buffer (never tracked by autograd)
         self.xn_var = xn_var       # the same values as an autograd variable when the caller wants dLoss/dx, else None
         self.T = T
-        self._pre = None
         self._stats = {}
 
     @property
@@ -125,17 +125,6 @@ class SeriesPack:
     @property
     def Tp(self):
         return self.xn.shape[2]
-
-    def prefix(self) -> Tuple[torch.Tensor, torch.Tensor]:
-        """Stand-alone fp64 prefix sums (ign_window_prefix); the distance kernels use window_stats() instead."""
-        if self._pre is None:
-            B, M, T = self.B, self.M, self.T
-            pre = torch.empty((2, B, M, C.lib.ign_prefix_pitch(T)), dtype=torch.float64, device=self.xn.device)
-            with torch.cuda.device(self.xn.device):
-                C.check(STATS.call("window_prefix", 1, lambda: C.lib.ign_window_prefix(
-                    _ptr(self.xn), _ptr(pre[0]), _ptr(pre[1]), B, M, T, _stream())), "ign_window_prefix")
-            self._pre = (pre[0], pre[1])
-        return self._pre
 
     def prepare_stats(self, dist: str, groups):
         """One fused prefix + window-difference pass for several (L, stride) groups (ign_window_stats).
@@ -245,31 +234,18 @@ def instance_norm(x: torch.Tensor) -> SeriesPack:
     return SeriesPack(xn, T)
 
 
-# When a model owns several length groups (ShapeBottleneckModel: four), the memory-bound preparation phase of every
-# group's backward (pooling backward, tie pre-check) CAN be issued on a side stream with only the compute-bound
-# contractions on the main stream, each waiting for its own group's event.  MEASURED ON B200 AND OFF BY DEFAULT: at
-# config 2 it changes nothing for the L1 engine (22.57 vs 22.55 ms per step: the contraction's three CTAs per SM leave
-# no shared memory for a pooling CTA to co-reside) and costs the tcgen05 engine 4 % (8.6 -> 8.95 ms: the persistent
-# one-CTA-per-SM contraction and the pooling kernel time-slice the SMs instead of overlapping).  IGN_OVERLAP_BWD_PREPARE=1
-# enables it for experiments; the deep expert's side stream (models/InterpGN.py) is the overlap that pays.
-OVERLAP_BWD_PREPARE = os.environ.get("IGN_OVERLAP_BWD_PREPARE", "0") == "1"
-_side_streams = {}
-
-
-def _side_stream(device):
-    key = str(device)
-    if key not in _side_streams:
-        _side_streams[key] = torch.cuda.Stream(device=device)
-    return _side_streams[key]
+# Has no effect; kept because bench.py saves and restores it around its per-kernel timing.
+OVERLAP_BWD_PREPARE = False
 
 
 class _Group:
     """One length group's forward state (what the backward needs)."""
-    __slots__ = ("desc", "dist", "pool", "stored", "thr_shape", "n_saved", "needs")   # needs: (any, W, threshold)
+    __slots__ = ("desc", "dist", "pool", "stored", "thr_shape", "needs")   # needs: (any, W, threshold)
 
 
 def _forward_group(pack: SeriesPack, W, threshold, stride, eps, dist, pool, precision, need_grad):
-    """Launch one group's forward.  Returns (group record, outputs (p, dmin, idx), tensors to save for backward)."""
+    """Launch one group's forward.  Returns (group record, outputs (p, dmin, idx), the 4 tensors or Nones to save for
+    backward)."""
     xn = pack.xn
     B, M, T, Tp = pack.B, pack.M, pack.T, pack.Tp
     K, M2, L = W.shape
@@ -301,49 +277,48 @@ def _forward_group(pack: SeriesPack, W, threshold, stride, eps, dist, pool, prec
     rec = _Group()
     rec.desc, rec.dist, rec.pool, rec.stored = desc, dist, pool, bool(store)
     rec.thr_shape = None if threshold is None else threshold.shape
-    saved = (Wc, out, idx, dstore if store else thr) if need_grad else ()
-    rec.n_saved = len(saved)
+    saved = (Wc, out, idx, dstore if store else thr) if need_grad else (None,) * 4
     return rec, (out[0], out[1], idx), saved
 
 
-def _backward_group_args(rec: _Group, pack: SeriesPack, saved, g_p, need_dthr):
-    """Host-side preparation of one group's backward: (g, dthr, call) where call(phases) launches the library."""
+def _backward_group(rec: _Group, pack: SeriesPack, saved, g_p, need_dx):
+    """Host side of one group's backward: returns (dW or None, dthreshold or None, launch or None).  launch(dxn)
+    allocates the group's workspace, runs the library (adding dLoss/dxn into dxn unless it is None) and releases the
+    workspace on return: every launch is on the current stream, so the next group gets the same block in stream order."""
     Wc, out, idx, extra = saved
     dstore, thr = (extra, None) if rec.stored else (None, extra)
     desc = rec.desc
+    _, need_w, need_thr = rec.needs
     g = g_p.to(torch.float32).contiguous()
     dthr = None
     if rec.pool == "lts_min":
         p = out[0]
         sig = p * (1.0 - p)                         # d sigmoid(thr - min_d)
-        if need_dthr:
+        if need_thr:
             dthr = (g * sig).sum(dim=0).reshape(rec.thr_shape)
         g = (-g * sig).contiguous()                 # dLoss/d(min_d)
+    if not need_w and not need_dx:
+        return None, dthr, None
     st0, st1 = pack.window_stats(rec.dist, desc.L, desc.stride)
     if rec.stored:
         nbytes = C.lib.ign_shapelet_backward_workspace(byref(desc))
     else:       # recompute mode: the library walks the shapelets in chunks inside this bounded workspace
         nbytes = C.lib.ign_shapelet_backward_recompute_workspace(byref(desc), STORE_BUDGET_BYTES)
-    ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=g.device)
-    dW = torch.empty_like(Wc)
+    dW = torch.empty_like(Wc) if need_w else None      # None: the library only prepares the coefficients for dxn
     tag = "shapelet_bwd/%s/L%d" % (rec.dist, desc.L)
     STATS.note_engine(tag, desc, True)
 
-    def call(phases):
+    def launch(dxn):
+        ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=g.device)
         with torch.cuda.device(g.device):
-            launch = lambda: C.lib.ign_shapelet_backward_phases(
+            C.check(STATS.call(tag, 2 if need_w else 1, lambda: C.lib.ign_shapelet_backward(
                 byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(thr), _ptr(g), _ptr(dstore),
-                _ptr(out[1]), _ptr(idx), _ptr(dW), _ptr(ws), int(nbytes), int(phases), _stream())
-            if phases == C.BWD_PREPARE:            # counted and timed with the contraction call of the same group
-                C.check(launch(), "ign_shapelet_backward_phases")
-            else:
-                C.check(STATS.call(tag, 2, launch), "ign_shapelet_backward")
-    def call_dx(dxn):      # after call(PREPARE): adds this group's dLoss/dxn (ign_shapelet_backward_input)
-        with torch.cuda.device(g.device):
-            C.check(STATS.call("shapelet_bwd_input/%s/L%d" % (rec.dist, desc.L), 1, lambda: C.lib.ign_shapelet_backward_input(
-                byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(dstore), _ptr(dxn), _ptr(ws),
-                int(nbytes), _stream())), "ign_shapelet_backward_input")
-    return dW, dthr, call, (g, ws, st0, st1), call_dx
+                _ptr(out[1]), _ptr(idx), _ptr(dW), _ptr(ws), int(nbytes), _stream())), "ign_shapelet_backward")
+            if dxn is not None:
+                C.check(STATS.call("shapelet_bwd_input/%s/L%d" % (rec.dist, desc.L), 1, lambda: C.lib.ign_shapelet_backward_input(
+                    byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(dstore), _ptr(dxn), _ptr(ws),
+                    int(nbytes), _stream())), "ign_shapelet_backward_input")
+    return dW, dthr, launch
 
 
 def shapelet_transform(pack: SeriesPack, W: torch.Tensor, stride: int = 1, eps: float = 1.0, dist: str = "l1",
@@ -362,9 +337,8 @@ def shapelet_transform(pack: SeriesPack, W: torch.Tensor, stride: int = 1, eps: 
 
 
 class _SbmTransform(torch.autograd.Function):
-    """All length groups of a ShapeBottleneckModel as ONE autograd node (the python loop of Shapelet.py:191-194): same
-    kernels as _ShapeletTransform per group, but the backward sees every group's upstream gradient at once and can
-    pipeline the groups' preparation phases against the contractions (see OVERLAP_BWD_PREPARE)."""
+    """All length groups of a ShapeBottleneckModel as ONE autograd node (the python loop of Shapelet.py:191-194).  The
+    backward launches the groups one after another, each with its own workspace (_backward_group)."""
 
     @staticmethod
     def forward(ctx, pack: SeriesPack, cfgs, track, xn_var, *params):      # params = W_0, thr_0, W_1, thr_1, ...
@@ -395,50 +369,25 @@ class _SbmTransform(torch.autograd.Function):
         recs, pack = ctx.recs, ctx.pack
         saved = ctx.saved_tensors
         grads = [None] * (2 * len(recs))
-        jobs, keep, off = [], [], 0
+        launches = []
         for gi, rec in enumerate(recs):
-            sv = saved[off:off + rec.n_saved]
-            off += rec.n_saved
             g_p, g_dmin = gs[3 * gi], gs[3 * gi + 1]
             if g_dmin is not None:
                 raise NotImplementedError("ign_b200: gradient through the reported min distance is not implemented")
             if g_p is None or not rec.needs[0]:
                 continue
-            dW, dthr, call, k, call_dx = _backward_group_args(rec, pack, sv, g_p, rec.needs[2])
-            keep.append(k)
-            grads[2 * gi + 1] = dthr
-            if rec.needs[1]:
-                grads[2 * gi] = dW
-            if rec.needs[1] or ctx.need_dx:
-                jobs.append((rec, call, call_dx, rec.needs[1]))
-        dxn = None
-        if ctx.need_dx:          # input gradients (saliency): per group the pooling backward, then dLoss/dxn from its coefficients
-            dxn = torch.zeros_like(pack.xn)
-            for rec, call, call_dx, want_w in jobs:
-                call((C.BWD_PREPARE | C.BWD_CONTRACT) if want_w else C.BWD_PREPARE)
-                call_dx(dxn)
-            return (None, None, None, dxn) + tuple(grads)
-        jobs = [(rec, call) for rec, call, _, _ in jobs]
-        split = OVERLAP_BWD_PREPARE and len(jobs) > 1 and all(rec.stored for rec, _ in jobs)
-        if not split:
-            for _, call in jobs:
-                call(C.BWD_PREPARE | C.BWD_CONTRACT)
-        else:
-            dev = pack.xn.device
-            cur, side = torch.cuda.current_stream(dev), _side_stream(dev)
-            side.wait_stream(cur)                          # upstream gradients and workspaces are ready
-            events = []
-            with torch.cuda.stream(side):
-                for _, call in jobs:
-                    call(C.BWD_PREPARE)
-                    ev = torch.cuda.Event()
-                    ev.record(side)
-                    events.append(ev)
-            for (_, call), ev in zip(jobs, events):
-                cur.wait_event(ev)                         # this group's coefficients (and tie flags) are written
-                call(C.BWD_CONTRACT)
-            # every side-stream kernel precedes one of the waits above: the main stream is ordered after all of them
-        return (None, None, None, None) + tuple(grads)
+            grads[2 * gi], grads[2 * gi + 1], launch = _backward_group(rec, pack, saved[4 * gi:4 * gi + 4], g_p,
+                                                                       ctx.need_dx)
+            if launch is not None:
+                launches.append(launch)
+        # input gradients (saliency): each group adds dLoss/dxn from the coefficients its own backward call left
+        dxn = torch.zeros_like(pack.xn) if ctx.need_dx else None
+        # The host work of every group first, then the launches back to back, one workspace at a time.  Host work
+        # between the launches shifts how the shapelet kernels overlap the deep expert's side stream: measured at
+        # +0.3-0.6 % (L1) and +4 % (cosine / 3xTF32) per step at config 2 on a B200 at 1000 W, with the same kernel times.
+        for launch in launches:
+            launch(dxn)
+        return (None, None, None, dxn) + tuple(grads)
 
 
 def sbm_transform(pack: SeriesPack, layers):

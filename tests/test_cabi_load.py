@@ -17,9 +17,9 @@ def declared_functions():
     return sorted(set(re.findall(r"\b(ign_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_header_declares_expected_surface():
+def test_header_declares_abi3_surface():
     names = declared_functions()
-    for n in ("ign_instnorm_forward", "ign_window_prefix", "ign_shapelet_forward", "ign_shapelet_backward",
+    for n in ("ign_instnorm_forward", "ign_window_stats", "ign_shapelet_forward", "ign_shapelet_backward",
               "ign_gate_forward", "ign_gate_backward", "ign_sbm_transform_host", "ign_last_error"):
         assert n in names
 
@@ -33,11 +33,11 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), "libign_b200.so does not export %s" % name
 
 
-def test_binding_covers_header_and_fails_loudly_without_gpu():
+def test_binding_covers_abi3_header_and_fails_loudly_without_gpu():
     import torch
     from layers import ign_cabi as C
     assert C.exported_symbols() == declared_functions()
-    assert C.lib.ign_abi_version() == 2 == C.IGN_ABI_VERSION
+    assert C.lib.ign_abi_version() == 3 == C.IGN_ABI_VERSION
     assert C.padded_len(1000) == 1000 and C.padded_len(29) == 32
     assert C.num_windows(1000, 100, 1) == 901 and C.num_windows(4000, 400, 8) == 451
     assert C.num_windows(5, 6, 1) == 0

@@ -54,7 +54,7 @@ def test_instnorm_cluster_kernel_geometries():
         assert float(pack.xn[:, 0, :].abs().max()) == 0.0
 
 
-def test_instnorm_and_prefix_kernels():
+def test_instnorm_and_window_stats_kernels():
     from layers.shapelet_ops import instance_norm
     torch.manual_seed(3)
     for (B, T, M) in [(3, 29, 12), (2, 1000, 125), (4, 130, 33), (2, 4100, 5), (1, 257, 16)]:
@@ -63,15 +63,10 @@ def test_instnorm_and_prefix_kernels():
         ref = O.instance_norm(x)
         torch.testing.assert_close(pack.xn[:, :, :T].cpu(), ref, rtol=2e-5, atol=2e-6)
         assert float(pack.xn[:, :, T:].abs().sum()) == 0.0
-        p1, p2 = pack.prefix()
-        own = pack.xn[:, :, :T].double().cpu()       # prefix sums are defined on the kernel's own xn
+        own = pack.xn[:, :, :T].double().cpu()       # window statistics are defined on the kernel's own xn
         r1 = torch.cumsum(own, -1)
         r2 = torch.cumsum(own ** 2, -1)
-        # row layout: slot 3 holds P[0] = 0, slot 4+j holds P[j+1] (include/ign_b200.h)
-        torch.testing.assert_close(p1[:, :, 4:4 + T].cpu(), r1, rtol=1e-9, atol=1e-9)
-        torch.testing.assert_close(p2[:, :, 4:4 + T].cpu(), r2, rtol=1e-9, atol=1e-9)
-        assert float(p1[:, :, :4].abs().sum()) == 0.0 and float(p2[:, :, :4].abs().sum()) == 0.0
-        # fused per-group window statistics against the same prefix sums
+        # fused per-group window statistics against fp64 prefix sums
         L, s = max(3, T // 5), 1 if T < 3000 else 7
         Tw = (T - L) // s + 1
         j0 = torch.arange(Tw) * s

@@ -548,6 +548,44 @@ def test_recompute_backward_at_k1000_bounded_workspace(tiny_store_budget):
     assert_close(dW, dW_ref, 1e-4, 1e-4 * float(dW_ref.abs().max()), "K=1000 recompute dW")
 
 
+@pytest.mark.parametrize("mode", ["stored", "recompute"])
+def test_backward_holds_one_group_workspace_at_a_time(tiny_store_budget, mode):
+    """Four length groups as one autograd node (sbm_transform, as ShapeBottleneckModel runs them): the backward allocates
+    each group's workspace just before that group's call and releases it after, so the memory it adds is one workspace
+    plus the gradients, not the sum of the four workspaces."""
+    from ctypes import byref
+    from layers import ign_cabi as C
+    from layers.shapelet_ops import SeriesPack, sbm_transform
+    from models.Shapelet import Shapelet
+    B, M, T, K, Ls = 64, 16, 1000, 16, (50, 100, 150, 200)
+    descs = [C.ShapeletDesc(B, M, T, C.padded_len(T), K, L, 1, 1.0, C.DIST["l1"], C.POOL["rbf_max"], C.PRECISION["fp32"])
+             for L in Ls]
+    dstore = [int(C.lib.ign_shapelet_dstore_bytes(byref(d))) for d in descs]
+    if mode == "stored":
+        ws = [int(C.lib.ign_shapelet_backward_workspace(byref(d))) for d in descs]
+    else:
+        budget = 3 * max(dstore) // 2
+        assert all(2 * n > budget for n in dstore)          # every group takes the recompute backward
+        tiny_store_budget(budget)
+        ws = [int(C.lib.ign_shapelet_backward_recompute_workspace(byref(d), budget)) for d in descs]
+    assert max(ws) < 1.5 * min(ws)                          # similar sizes: one workspace is well below their sum
+    torch.manual_seed(41)
+    layers = [Shapelet(M, L, K).to(DEV) for L in Ls]
+    pack = SeriesPack.from_channel_major(torch.randn(B, M, T, device=DEV))
+    gs = [torch.randn(B, K, M, device=DEV) for _ in Ls]
+    loss = sum((p * g).sum() for (p, _, _), g in zip(sbm_transform(pack, layers), gs))
+    torch.cuda.synchronize()
+    base = torch.cuda.memory_allocated()
+    torch.cuda.reset_peak_memory_stats()
+    loss.backward()
+    torch.cuda.synchronize()
+    peak = torch.cuda.max_memory_allocated() - base
+    grads = sum(4 * K * M * L + 4 * B * K * M for L in Ls)     # dW and the upstream dLoss/dp of every group
+    assert peak < max(ws) + grads + 2 * 2 ** 20, (peak, ws)
+    assert peak < sum(ws), (peak, ws)
+    assert all(float(layer.weights.grad.abs().sum()) > 0 for layer in layers)
+
+
 def test_engine_report_matches_what_runs():
     """ign_shapelet_engine is what bench.py / tools/sweep.py label their rows with."""
     from layers.shapelet_ops import STATS

@@ -198,10 +198,8 @@ def test_full_size_model_matches_live_reference_golden(name, precision, rtol, at
                 assert_close(got, ref, 10 * gtol, gtol * float(ref.abs().max()), tag + " sampled grad " + k)
 
 
-def test_pipelined_backward_phases_give_identical_gradients(monkeypatch):
-    """ign_shapelet_backward_phases (PREPARE on a side stream, CONTRACT on the main stream, per-group events) is the same
-    arithmetic in a different launch order: bit-identical gradients, with and without the deep expert's side stream."""
-    from layers import shapelet_ops
+def test_overlapped_experts_give_identical_gradients():
+    """The deep expert on its side stream is the same arithmetic as on the main stream: bit-identical gradients."""
     model, g = build("model_small_chisco")
     x, y = t(g["x"], DEV), torch.as_tensor(g["y"]).to(DEV)
 
@@ -213,13 +211,12 @@ def test_pipelined_backward_phases_give_identical_gradients(monkeypatch):
         torch.cuda.synchronize()
         return [p.grad.clone() for p in model.sbm.parameters()]
 
-    base = grads()
-    monkeypatch.setattr(shapelet_ops, "OVERLAP_BWD_PREPARE", True)
-    piped = grads()
+    model.overlap_experts = True
+    overlapped = grads()
     model.overlap_experts = False
     serial = grads()
-    for a, b, c in zip(base, piped, serial):
-        assert torch.equal(a, b) and torch.equal(a, c)
+    for a, b in zip(overlapped, serial):
+        assert torch.equal(a, b)
 
 
 @pytest.mark.parametrize("name", ["model_jv_interpgn", "model_jv_interpgn_cos", "model_small_chisco"])
