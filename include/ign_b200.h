@@ -177,6 +177,23 @@ int32_t ign_shapelet_backward(const ign_shapelet_desc* desc, const float* xn_dev
                               const int32_t* argmin_dev, float* dW_dev, void* workspace_dev,
                               size_t workspace_bytes, void* stream);
 
+/* ign_shapelet_backward with a gradient on the second output as well, min_t d (dmin_dev of the forward,
+ * Shapelet.py:84 | :111), for losses that use it (ShapeBottleneckModel's ModelInfo.d):
+ *   gdmin_dev [B,K,M] = dLoss/d(min_t d), or NULL (exactly ign_shapelet_backward, which forwards here with NULL).
+ * min_t d is the hard minimum in both poolings, so gdmin_dev[b,k,m] is added to the coefficient of ONE window,
+ * argmin_t d with the first index on ties — the forward's argmin_dev.  For rbf_max that is not always the window the
+ * straight-through arg-max of p picks (where every p underflows to 0 the arg-max is window 0).
+ *   Stored-distance mode: argmin_dev is required whenever gdmin_dev is given (for rbf_max too).  Recompute mode: the
+ *   index is recomputed with the distances; argmin_dev is not read.
+ *   g_dev stays required: pass zeros when only min_t d carries a gradient.
+ * Every other argument, the workspace and the dW_dev == NULL case are as for ign_shapelet_backward, and
+ * ign_shapelet_backward_input then gives the input gradient of both outputs. */
+int32_t ign_shapelet_backward_dmin(const ign_shapelet_desc* desc, const float* xn_dev, const float* st0_dev,
+                                   const float* st1_dev, const float* W_dev, const float* threshold_dev,
+                                   const float* g_dev, const float* gdmin_dev, const float* dstore_dev,
+                                   const float* dmin_dev, const int32_t* argmin_dev, float* dW_dev,
+                                   void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* Gradient w.r.t. the normalised input series — what autograd gives a user of the reference who asks for input
  * gradients (saliency, gradcheck) through Shapelet.forward; the training loop never does
  * (experiment_classification.py:315).  Call AFTER ign_shapelet_backward (with or without dW_dev) of the same group

@@ -178,10 +178,10 @@ size_t ign_shapelet_backward_recompute_workspace(const ign_shapelet_desc* d, siz
   return shapelet_bwd_recompute_workspace(*d, budget_bytes);
 }
 
-int32_t ign_shapelet_backward(const ign_shapelet_desc* d, const float* xn, const float* st0, const float* st1,
-                              const float* W, const float* thr, const float* g, const float* dstore,
-                              const float* dmin, const int32_t* argmin, float* dW, void* ws, size_t ws_bytes,
-                              void* stream) {
+int32_t ign_shapelet_backward_dmin(const ign_shapelet_desc* d, const float* xn, const float* st0, const float* st1,
+                                   const float* W, const float* thr, const float* g, const float* gdmin,
+                                   const float* dstore, const float* dmin, const int32_t* argmin, float* dW, void* ws,
+                                   size_t ws_bytes, void* stream) {
   int rc = check_desc(d, "shapelet_backward");
   if (rc) return rc;
   IGN_REQUIRE(xn && W && g && ws, "shapelet_backward: null pointer");
@@ -190,11 +190,19 @@ int32_t ign_shapelet_backward(const ign_shapelet_desc* d, const float* xn, const
   if (!dstore) {   // recompute mode: nothing was kept by the forward
     IGN_REQUIRE(dW, "shapelet_backward(recompute): dW is required (dW == NULL needs the stored distances)");
     IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || thr, "shapelet_backward(recompute): lts_min needs the threshold again");
-    return launch_shapelet_bwd_recompute(*d, xn, st0, st1, W, thr, g, dW, ws, ws_bytes, (cudaStream_t)stream);
+    return launch_shapelet_bwd_recompute(*d, xn, st0, st1, W, thr, g, gdmin, dW, ws, ws_bytes, (cudaStream_t)stream);
   }
   IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || (dmin && argmin), "shapelet_backward: lts_min needs the forward's dmin and argmin");
-  return launch_shapelet_bwd_simt(*d, xn, st0, st1, W, g, d->K, 0, dstore, dmin, argmin, dW, ws, ws_bytes,
+  IGN_REQUIRE(!gdmin || argmin, "shapelet_backward: gdmin needs the forward's argmin (the window it lands on)");
+  return launch_shapelet_bwd_simt(*d, xn, st0, st1, W, g, gdmin, d->K, 0, dstore, dmin, argmin, dW, ws, ws_bytes,
                                   (cudaStream_t)stream);
+}
+
+int32_t ign_shapelet_backward(const ign_shapelet_desc* d, const float* xn, const float* st0, const float* st1,
+                              const float* W, const float* thr, const float* g, const float* dstore,
+                              const float* dmin, const int32_t* argmin, float* dW, void* ws, size_t ws_bytes,
+                              void* stream) {
+  return ign_shapelet_backward_dmin(d, xn, st0, st1, W, thr, g, nullptr, dstore, dmin, argmin, dW, ws, ws_bytes, stream);
 }
 
 int32_t ign_shapelet_backward_input(const ign_shapelet_desc* d, const float* xn, const float* st0, const float* st1,

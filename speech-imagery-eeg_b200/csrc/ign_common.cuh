@@ -48,20 +48,21 @@ int launch_shapelet_fwd_simt(const ign_shapelet_desc& d, const float* xn, const 
                              const float* W, const float* thr, float* p, float* dmin,
                              int* argmin, float* dstore, cudaStream_t st);
 size_t shapelet_bwd_workspace_simt(const ign_shapelet_desc& d);
-// g [B,gK,M]: the launch's K shapelets are gk0 .. gk0+K-1 of it; dstore == NULL: the distances sit in the coefficient
-// buffer of the workspace already (recompute mode) and are converted in place; dW == NULL: the preparation alone (the
-// coefficients for launch_shapelet_dx), no contraction
+// g [B,gK,M]: the launch's K shapelets are gk0 .. gk0+K-1 of it; gdmin: NULL, or dLoss/d(min_t d) indexed like g (it
+// is added at the window argmin names); dstore == NULL: the distances sit in the coefficient buffer of the workspace
+// already (recompute mode) and are converted in place; dW == NULL: the preparation alone (the coefficients for
+// launch_shapelet_dx), no contraction
 int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const float* st0,
-                             const float* st1, const float* W, const float* g, int gK, int gk0, const float* dstore,
-                             const float* dmin, const int* argmin, float* dW, void* ws, size_t ws_bytes,
-                             cudaStream_t st);
+                             const float* st1, const float* W, const float* g, const float* gdmin, int gK, int gk0,
+                             const float* dstore, const float* dmin, const int* argmin, float* dW, void* ws,
+                             size_t ws_bytes, cudaStream_t st);
 bool shapelet_bwd_coef_offset(const ign_shapelet_desc& d, size_t* off_floats, size_t* total_bytes);
 int launch_shapelet_dx(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1, const float* W,
                        const float* coef, const float* dstore, float* dxn, cudaStream_t st);
 size_t shapelet_bwd_recompute_workspace(const ign_shapelet_desc& d, size_t budget);
 int launch_shapelet_bwd_recompute(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1,
-                                  const float* W, const float* thr, const float* g, float* dW, void* ws,
-                                  size_t ws_bytes, cudaStream_t st);
+                                  const float* W, const float* thr, const float* g, const float* gdmin, float* dW,
+                                  void* ws, size_t ws_bytes, cudaStream_t st);
 // engine selection + launch shared by ign_shapelet_forward and the recompute backward (api.cu)
 size_t shapelet_forward_workspace_bytes(const ign_shapelet_desc& d);
 int shapelet_forward_dispatch(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* W,

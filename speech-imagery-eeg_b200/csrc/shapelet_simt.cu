@@ -104,6 +104,7 @@ struct PoolArgs {
   const float* st0; const float* st1; int SP; const float* wstat;   // window stats [B,M,SP]; wstat [K][M]: sum (w-mean)^2 (pearson)
   float* coef;          // [B][M][K][Ts]
   float* rowsc;         // [B][M][K][2] per-row scalars for the finalize kernel
+  const float* gd;      // NULL, or dLoss/d(min_t d) [B,gK,M] indexed like g: added at the window `argmin` names
 };
 
 
@@ -500,6 +501,10 @@ __device__ __forceinline__ unsigned hash_slot(unsigned key, unsigned mask) {
 // hard one-hot = first arg-max of p, Shapelet.py:79 | for lts_min the forward's argmin, :105), then the
 // coefficient a_t = dLoss/dd_t times the distance mode's norm factor, written to `coef`; two per-row
 // scalars go to `rowsc` for the finalize kernel.
+// GD (a.gd != NULL): the layer's second output min_t d (Shapelet.py:84 | :111) has a gradient too.  It is the hard min,
+// so its whole gradient lands on ONE window, the forward's argmin (first index on ties) — for rbf_max not necessarily
+// the arg-max of p that the straight-through one-hot selects (every p underflows to 0: arg-max 0, the min elsewhere).
+// The training path never differentiates it and runs the GD = false instantiations, which are the kernels without it.
 __device__ __forceinline__ void cp_async16_pool(void* dst, const void* src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
 }
@@ -510,7 +515,13 @@ __device__ __forceinline__ void cp_async16_pool(void* dst, const void* src) {
 template <int DIST>
 __device__ __forceinline__ float pool_emit(float c, float d, float s0, float s1, float wst, float& sc0, float& sc1);
 
-template <int POOL, int DIST>
+// c0..c3, the coefficients of windows t0 .. t0+3: + v on window i (nothing when i is outside them)
+__device__ __forceinline__ void add_at4(float& c0, float& c1, float& c2, float& c3, int i, int t0, float v) {
+  const int h = i - t0;
+  if ((unsigned)h < 4u) { c0 += h == 0 ? v : 0.f; c1 += h == 1 ? v : 0.f; c2 += h == 2 ? v : 0.f; c3 += h == 3 ? v : 0.f; }
+}
+
+template <int POOL, int DIST, bool GD>
 __global__ void __launch_bounds__(256) pool_bwd_kernel(const Geo g, const PoolArgs a, int rows) {
   extern __shared__ __align__(16) float prow[];          // [warps][2][DP]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
@@ -540,6 +551,9 @@ __global__ void __launch_bounds__(256) pool_bwd_kernel(const Geo g, const PoolAr
   float Zs = 0.f, S1s = 0.f, shift = 0.f;
   int ih;
   if (POOL == IGN_POOL_LTS_MIN) { shift = a.dmin[o]; ih = a.argmin[o]; }
+  float gdv = 0.f;
+  int idm = -1;
+  if (GD) { gdv = a.gd[((size_t)b * a.gK + a.gk0 + k) * g.M + m]; idm = a.argmin[o]; }
   __syncwarp();
   // Both passes walk the row in float4 chunks (lane owns chunks lane, lane + 32, ...): 128-bit shared-memory reads and
   // global stores, and in pass 2 the window-statistics loads of kPoolUnroll chunks are issued before any of them is
@@ -608,6 +622,7 @@ __global__ void __launch_bounds__(256) pool_bwd_kernel(const Geo g, const PoolAr
       const float soft = fast_ex2((shift - d) * kLog2e) * invZ;
       c = gk * fmaf(-soft, d - bar, t == ih ? 1.f : 0.f);
     }
+    if (GD && t == idm) c += gdv;
     return pool_emit<DIST>(c, d, sxn, mu, wst, sc0, sc1);
   };
   constexpr bool kS0 = DIST == IGN_DIST_COSINE || DIST == IGN_DIST_PEARSON;
@@ -656,7 +671,7 @@ __global__ void __launch_bounds__(256) pool_bwd_kernel(const Geo g, const PoolAr
 // configs below T = 2000).  The generic kernel above spends 37 issue slots per element — two passes that each
 // evaluate both exponentials — and is issue-bound at 65 % of HBM peak.  Here each lane owns NCH float4 chunks of the
 // row; pass 1 evaluates the exponentials once and keeps (U_t, V_t) in registers with
-//     c_t = Kc * U_t * (V_t - vbar) + [t == ih] * fix
+//     c_t = Kc * U_t * (V_t - vbar) + [t == ih] * fix  (+ [t == argmin] * gd when GD)
 //   rbf_max: V = p' = log2(e) p_t,  U = e^{p_t} p' d_t,  vbar = sum(e^p p')/Z,  Kc = -2 eps^2 g / (Z log2(e)^2),  fix = -2 eps^2 g p_ih d_ih
 //   lts_min: V = d_t,  U = e^{dmin - d_t},  vbar = sum(U d)/Z,  Kc = -g/Z,  fix = g
 // so pass 2 is three FP32 instructions per element over registers, all shared-memory and global accesses are
@@ -694,7 +709,7 @@ __device__ __forceinline__ float pool_emit(float c, float d, float s0, float s1,
 // than contiguous ranges when nothing is reused).
 constexpr int pool_reg_min_blocks(int NCH) { return NCH <= 4 ? 3 : 2; }   // short rows are latency-bound: a third CTA per SM
 
-template <int POOL, int DIST, int NCH>
+template <int POOL, int DIST, int NCH, bool GD>
 __global__ void __launch_bounds__(256, pool_reg_min_blocks(NCH)) pool_bwd_reg_kernel(const Geo g, const PoolArgs a, int rows) {
   extern __shared__ __align__(16) float prow[];          // [warps][kPoolStages][DP]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
@@ -741,6 +756,9 @@ __global__ void __launch_bounds__(256, pool_reg_min_blocks(NCH)) pool_bwd_reg_ke
     float sl2 = 0.f;
     int ih = 0;
     if (POOL == IGN_POOL_LTS_MIN) { sl2 = a.dmin[o] * kLog2e; ih = a.argmin[o]; }
+    float gdv = 0.f;                                       // GD: + gdv on window idm (the forward's argmin)
+    int idm = -1;
+    if (GD) { gdv = a.gd[((size_t)b * a.gK + a.gk0 + k) * g.M + m]; idm = a.argmin[o]; }
 
     // ---- pass 1: exponentials once, (U, V) to registers, soft-max statistics, chunk-wise arg-max
     float4 U[NCH], V[NCH];
@@ -849,6 +867,7 @@ __global__ void __launch_bounds__(256, pool_reg_min_blocks(NCH)) pool_bwd_reg_ke
         if ((unsigned)hc < 4u) {
           c0 += hc == 0 ? fix : 0.f; c1 += hc == 1 ? fix : 0.f; c2 += hc == 2 ? fix : 0.f; c3 += hc == 3 ? fix : 0.f;
         }
+        if (GD) add_at4(c0, c1, c2, c3, idm, t0, gdv);
         float4 d = make_float4(0.f, 0.f, 0.f, 0.f), s0 = d, s1 = d;
         if (kStats) d = d4[j * 32 + lane];
         if (DIST == IGN_DIST_COSINE) s0 = S[j < NS ? j : 0];
@@ -867,6 +886,7 @@ __global__ void __launch_bounds__(256, pool_reg_min_blocks(NCH)) pool_bwd_reg_ke
       const int t = tt + (S) * 32;                                                             \
       float c = Kc * UC * (VC - vbar);                                                         \
       if (t == ih) c += fix;                                                                   \
+      if (GD && t == idm) c += gdv;                                                            \
       dst[t] = pool_emit<DIST>(c, kStats ? dr[t] : 0.f, kStats ? s0r[t] : 0.f,                 \
                                DIST == IGN_DIST_PEARSON ? s1r[t] : 0.f, wst, sc0, sc1);        \
     }
@@ -882,6 +902,7 @@ __global__ void __launch_bounds__(256, pool_reg_min_blocks(NCH)) pool_bwd_reg_ke
       if ((unsigned)hc < 4u) {
         cc[0] += hc == 0 ? fix : 0.f; cc[1] += hc == 1 ? fix : 0.f; cc[2] += hc == 2 ? fix : 0.f; cc[3] += hc == 3 ? fix : 0.f;
       }
+      if (GD) add_at4(cc[0], cc[1], cc[2], cc[3], idm, tv0, gdv);
       float4 d = make_float4(0.f, 0.f, 0.f, 0.f), s0 = d, s1 = d;
       if (kStats) d = d4[nfull * 32 + lane];
       if (DIST == IGN_DIST_COSINE) s0 = S[NS - 1];
@@ -1572,9 +1593,9 @@ size_t shapelet_bwd_workspace_simt(const ign_shapelet_desc& d) {
 }
 
 int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const float* st0,
-                             const float* st1, const float* W, const float* gr, int gK, int gk0, const float* dstore,
-                             const float* dmin, const int* argmin, float* dW, void* ws, size_t ws_bytes,
-                             cudaStream_t st) {
+                             const float* st1, const float* W, const float* gr, const float* gdmin, int gK, int gk0,
+                             const float* dstore, const float* dmin, const int* argmin, float* dW, void* ws,
+                             size_t ws_bytes, cudaStream_t st) {
   Geo g; BwdPlan bp;
   if (!base_geo(d, g)) { set_error("shapelet_backward: T=%d < L=%d", d.T, d.L); return IGN_ERR_INVALID; }
   if (!plan_bwd(g, bp)) { set_error("shapelet_backward: problem does not fit shared memory (T=%d L=%d)", d.T, d.L); return IGN_ERR_UNSUPPORTED; }
@@ -1596,7 +1617,7 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
     const int rows = d.B * d.M * d.K;
     // recompute mode passes dstore == NULL: the distances were just recomputed INTO the coefficient buffer and are
     // converted in place (every row is read into shared memory / registers by its own warp before it is rewritten)
-    PoolArgs pa{gr, gK, gk0, dstore ? dstore : base + wo.coef, dmin, argmin, st0, st1, stats_pitch(d.T, d.L, d.stride), base + wo.wstat, base + wo.coef, base + wo.rowsc};
+    PoolArgs pa{gr, gK, gk0, dstore ? dstore : base + wo.coef, dmin, argmin, st0, st1, stats_pitch(d.T, d.L, d.stride), base + wo.wstat, base + wo.coef, base + wo.rowsc, gdmin};
     const bool in_regs = g.Tw <= 1024;       // rows that fit NCH float4 chunks per lane (pool_bwd_reg_kernel)
     int warps = 8;
     const int stages = in_regs ? kPoolStages : 2;
@@ -1610,12 +1631,14 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
 #define IGN_POOL_LAUNCH_K(KERN)                                                         \
     { int rc = set_smem(KERN, smem); if (rc) return rc;                                 \
       KERN<<<pgrid, pblock, smem, st>>>(g, pa, rows); }
+#define IGN_POOL_LAUNCH_G(PV, DV, GV)                                                   \
+    { if (!in_regs) IGN_POOL_LAUNCH_K((pool_bwd_kernel<PV, DV, GV>))                    \
+      else if (g.Tw > 768) IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 8, GV>))      \
+      else if (g.Tw > 512) IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 6, GV>))      \
+      else if (g.Tw > 256) IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 4, GV>))      \
+      else IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 2, GV>)) }
 #define IGN_POOL_LAUNCH(PV, DV)                                                         \
-    { if (!in_regs) IGN_POOL_LAUNCH_K((pool_bwd_kernel<PV, DV>))                        \
-      else if (g.Tw > 768) IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 8>))          \
-      else if (g.Tw > 512) IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 6>))          \
-      else if (g.Tw > 256) IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 4>))          \
-      else IGN_POOL_LAUNCH_K((pool_bwd_reg_kernel<PV, DV, 2>)) }
+    { if (gdmin) IGN_POOL_LAUNCH_G(PV, DV, true) else IGN_POOL_LAUNCH_G(PV, DV, false) }
     if (d.pool == IGN_POOL_RBF_MAX) {
       switch (d.dist) {
         case IGN_DIST_L1: IGN_POOL_LAUNCH(IGN_POOL_RBF_MAX, IGN_DIST_L1) break;
@@ -1628,6 +1651,7 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
       else IGN_POOL_LAUNCH(IGN_POOL_LTS_MIN, IGN_DIST_SQL2)
     }
 #undef IGN_POOL_LAUNCH
+#undef IGN_POOL_LAUNCH_G
 #undef IGN_POOL_LAUNCH_K
     IGN_CUDA(cudaGetLastError());
   }
@@ -1720,8 +1744,8 @@ size_t shapelet_bwd_recompute_workspace(const ign_shapelet_desc& d, size_t budge
 }
 
 int launch_shapelet_bwd_recompute(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1,
-                                  const float* W, const float* thr, const float* gr, float* dW, void* ws,
-                                  size_t ws_bytes, cudaStream_t st) {
+                                  const float* W, const float* thr, const float* gr, const float* gdmin, float* dW,
+                                  void* ws, size_t ws_bytes, cudaStream_t st) {
   if (((uintptr_t)ws & 127) != 0) { set_error("shapelet_backward(recompute): workspace must be 128-byte aligned"); return IGN_ERR_INVALID; }
   const int Kc = recompute_chunk(d, ws_bytes);
   RecomputeLayout r;
@@ -1744,8 +1768,9 @@ int launch_shapelet_bwd_recompute(const ign_shapelet_desc& d, const float* xn, c
     int rc1 = shapelet_forward_dispatch(dc, xn, st0, W + wofs, thr ? thr + (size_t)k0 * d.M : nullptr, outp, outp + no,
                                         reinterpret_cast<int*>(outp + 2 * no), dbuf, base8 + rc.fws_off, rc.fws_bytes, st);
     if (rc1) return rc1;
-    // 2. pooling backward in place, contraction, finalize -> dW[k0 .. k0+Kc)
-    rc1 = launch_shapelet_bwd_simt(dc, xn, st0, st1, W + wofs, gr, d.K, k0, nullptr, outp + no,
+    // 2. pooling backward in place, contraction, finalize -> dW[k0 .. k0+Kc); gdmin is read like gr, at the chunk's
+    //    shapelets, and lands on the recomputed argmin of the chunk (the same kernels give the forward's index)
+    rc1 = launch_shapelet_bwd_simt(dc, xn, st0, st1, W + wofs, gr, gdmin, d.K, k0, nullptr, outp + no,
                                    reinterpret_cast<const int*>(outp + 2 * no), dW + wofs, ws, rc.bwd_bytes, st);
     if (rc1) return rc1;
   }

@@ -281,17 +281,20 @@ def _forward_group(pack: SeriesPack, W, threshold, stride, eps, dist, pool, prec
     return rec, (out[0], out[1], idx), saved
 
 
-def _backward_group(rec: _Group, pack: SeriesPack, saved, g_p, need_dx):
+def _backward_group(rec: _Group, pack: SeriesPack, saved, g_p, g_dmin, need_dx):
     """Host side of one group's backward: returns (dW or None, dthreshold or None, launch or None).  launch(dxn)
     allocates the group's workspace, runs the library (adding dLoss/dxn into dxn unless it is None) and releases the
-    workspace on return: every launch is on the current stream, so the next group gets the same block in stream order."""
+    workspace on return: every launch is on the current stream, so the next group gets the same block in stream order.
+    g_p or g_dmin may be None (no gradient on that output), not both."""
     Wc, out, idx, extra = saved
     dstore, thr = (extra, None) if rec.stored else (None, extra)
     desc = rec.desc
     _, need_w, need_thr = rec.needs
-    g = g_p.to(torch.float32).contiguous()
+    # min_t d is the hard minimum (Shapelet.py:84 | :111): its gradient goes to the argmin window, inside the library
+    gd = None if g_dmin is None else g_dmin.to(torch.float32).contiguous()
+    g = torch.zeros_like(out[0]) if g_p is None else g_p.to(torch.float32).contiguous()
     dthr = None
-    if rec.pool == "lts_min":
+    if rec.pool == "lts_min" and g_p is not None:     # min_t d does not depend on the threshold
         p = out[0]
         sig = p * (1.0 - p)                         # d sigmoid(thr - min_d)
         if need_thr:
@@ -310,10 +313,15 @@ def _backward_group(rec: _Group, pack: SeriesPack, saved, g_p, need_dx):
 
     def launch(dxn):
         ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=g.device)
+        head = (byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(thr), _ptr(g))
+        tail = (_ptr(dstore), _ptr(out[1]), _ptr(idx), _ptr(dW), _ptr(ws), int(nbytes), _stream())
         with torch.cuda.device(g.device):
-            C.check(STATS.call(tag, 2 if need_w else 1, lambda: C.lib.ign_shapelet_backward(
-                byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(thr), _ptr(g), _ptr(dstore),
-                _ptr(out[1]), _ptr(idx), _ptr(dW), _ptr(ws), int(nbytes), _stream())), "ign_shapelet_backward")
+            if gd is None:
+                C.check(STATS.call(tag, 2 if need_w else 1, lambda: C.lib.ign_shapelet_backward(*head, *tail)),
+                        "ign_shapelet_backward")
+            else:
+                C.check(STATS.call(tag, 2 if need_w else 1, lambda: C.lib.ign_shapelet_backward_dmin(
+                    *head, _ptr(gd), *tail)), "ign_shapelet_backward_dmin")
             if dxn is not None:
                 C.check(STATS.call("shapelet_bwd_input/%s/L%d" % (rec.dist, desc.L), 1, lambda: C.lib.ign_shapelet_backward_input(
                     byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(dstore), _ptr(dxn), _ptr(ws),
@@ -372,12 +380,10 @@ class _SbmTransform(torch.autograd.Function):
         launches = []
         for gi, rec in enumerate(recs):
             g_p, g_dmin = gs[3 * gi], gs[3 * gi + 1]
-            if g_dmin is not None:
-                raise NotImplementedError("ign_b200: gradient through the reported min distance is not implemented")
-            if g_p is None or not rec.needs[0]:
+            if (g_p is None and g_dmin is None) or not rec.needs[0]:
                 continue
             grads[2 * gi], grads[2 * gi + 1], launch = _backward_group(rec, pack, saved[4 * gi:4 * gi + 4], g_p,
-                                                                       ctx.need_dx)
+                                                                       g_dmin, ctx.need_dx)
             if launch is not None:
                 launches.append(launch)
         # input gradients (saliency): each group adds dLoss/dxn from the coefficients its own backward call left
