@@ -200,10 +200,34 @@ int32_t ign_shapelet_backward_dmin(const ign_shapelet_desc* desc, const float* x
  * with the same workspace: it reads the per-window coefficients that call left there.
  *   dxn_dev [B,M,Tp] += sum_k sum_t dLoss/dd[b,k,t] * d d_t / d xn[b,m,t*stride + l]     (ADDED: zero it once, call per group)
  * L1 (Shapelet.py:74, sign(0) = 0), cosine (:64-66), pearson (:11-19,:67-69).  SQL2: nothing is added — the
- * reference's ShapeletDistanceFunc.backward returns zeros for its input (Shapelet.py:40).  Stored-distance mode only. */
+ * reference's ShapeletDistanceFunc.backward returns zeros for its input (Shapelet.py:40).  Stored-distance mode only;
+ * recompute mode: ign_shapelet_backward_recompute_input below. */
 int32_t ign_shapelet_backward_input(const ign_shapelet_desc* desc, const float* xn_dev, const float* st0_dev,
                                     const float* st1_dev, const float* W_dev, const float* dstore_dev, float* dxn_dev,
                                     const void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* The input gradient in recompute mode, where no chunk's coefficients outlive the chunk: one call does what
+ * ign_shapelet_backward_dmin (dstore_dev == NULL) and ign_shapelet_backward_input do in the stored mode.  Per shapelet
+ * chunk it recomputes the window distances, runs the pooling backward, contracts into dW_dev (unless NULL) and adds
+ * the chunk's share of the input gradient into dxn_dev.  Each dxn row adds its shapelets in k order, chunk after
+ * chunk, as ign_shapelet_backward_input adds them in one pass.
+ *   g_dev / gdmin_dev (may be NULL) / threshold_dev (required for lts_min) as for ign_shapelet_backward_dmin.
+ *   dW_dev [K,M,L] is overwritten, or NULL when the weights are frozen: the contraction is skipped.
+ *   dxn_dev [B,M,Tp] += dLoss/dxn, as ign_shapelet_backward_input (ADDED; nothing for SQL2).
+ * The workspace (128-byte aligned, ign_shapelet_backward_recompute_input_workspace(desc, budget) bytes; the chunking
+ * is derived from workspace_bytes) holds, per chunk: the coefficient workspace of ign_shapelet_backward, the chunk's
+ * p / dmin / argmin, the forward's tcgen05 scratch and, for COSINE / PEARSON only, the chunk's window distances
+ * [B,M,Kc,Tw].  The input gradient of those two modes reads the distances after the pooling backward has turned them
+ * into coefficients, so they cannot be converted in place: at the same budget their chunks hold fewer shapelets than
+ * those of ign_shapelet_backward_recompute_workspace.  For L1 and SQL2 both queries return the same size.  At least
+ * one shapelet block, as for ign_shapelet_backward_recompute_workspace: the result can exceed a budget that is too
+ * small. */
+size_t ign_shapelet_backward_recompute_input_workspace(const ign_shapelet_desc* desc, size_t budget_bytes);
+int32_t ign_shapelet_backward_recompute_input(const ign_shapelet_desc* desc, const float* xn_dev, const float* st0_dev,
+                                              const float* st1_dev, const float* W_dev, const float* threshold_dev,
+                                              const float* g_dev, const float* gdmin_dev, float* dW_dev,
+                                              float* dxn_dev, void* workspace_dev, size_t workspace_bytes,
+                                              void* stream);
 
 /* InterpGN gate + mixture (InterpGN.py:44-52): q=softmax(s), eta=(C*sum q^2-1)/(C-1),
  * if use_gate: eta=1 where eta>gating_value; out=eta*s+(1-eta)*z.  s,z,out [B,C]; eta [B]. */

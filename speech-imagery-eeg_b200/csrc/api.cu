@@ -175,7 +175,12 @@ size_t ign_shapelet_dstore_bytes(const ign_shapelet_desc* d) {
 
 size_t ign_shapelet_backward_recompute_workspace(const ign_shapelet_desc* d, size_t budget_bytes) {
   if (check_desc(d, "shapelet_backward_recompute_workspace")) return 0;
-  return shapelet_bwd_recompute_workspace(*d, budget_bytes);
+  return shapelet_bwd_recompute_workspace(*d, budget_bytes, false);
+}
+
+size_t ign_shapelet_backward_recompute_input_workspace(const ign_shapelet_desc* d, size_t budget_bytes) {
+  if (check_desc(d, "shapelet_backward_recompute_input_workspace")) return 0;
+  return shapelet_bwd_recompute_workspace(*d, budget_bytes, true);
 }
 
 int32_t ign_shapelet_backward_dmin(const ign_shapelet_desc* d, const float* xn, const float* st0, const float* st1,
@@ -190,7 +195,8 @@ int32_t ign_shapelet_backward_dmin(const ign_shapelet_desc* d, const float* xn, 
   if (!dstore) {   // recompute mode: nothing was kept by the forward
     IGN_REQUIRE(dW, "shapelet_backward(recompute): dW is required (dW == NULL needs the stored distances)");
     IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || thr, "shapelet_backward(recompute): lts_min needs the threshold again");
-    return launch_shapelet_bwd_recompute(*d, xn, st0, st1, W, thr, g, gdmin, dW, ws, ws_bytes, (cudaStream_t)stream);
+    return launch_shapelet_bwd_recompute(*d, xn, st0, st1, W, thr, g, gdmin, dW, nullptr, ws, ws_bytes,
+                                         (cudaStream_t)stream);
   }
   IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || (dmin && argmin), "shapelet_backward: lts_min needs the forward's dmin and argmin");
   IGN_REQUIRE(!gdmin || argmin, "shapelet_backward: gdmin needs the forward's argmin (the window it lands on)");
@@ -218,6 +224,19 @@ int32_t ign_shapelet_backward_input(const ign_shapelet_desc* d, const float* xn,
   if (!shapelet_bwd_coef_offset(*d, &off, &total)) { set_error("shapelet_backward_input: T=%d < L=%d or the problem does not fit shared memory", d->T, d->L); return IGN_ERR_INVALID; }
   IGN_REQUIRE(ws_bytes >= total, "shapelet_backward_input: workspace %zu < %zu bytes (pass the workspace ign_shapelet_backward used)", ws_bytes, total);
   return launch_shapelet_dx(*d, xn, st0, st1, W, reinterpret_cast<const float*>(ws) + off, dstore, dxn, (cudaStream_t)stream);
+}
+
+int32_t ign_shapelet_backward_recompute_input(const ign_shapelet_desc* d, const float* xn, const float* st0,
+                                              const float* st1, const float* W, const float* thr, const float* g,
+                                              const float* gdmin, float* dW, float* dxn, void* ws, size_t ws_bytes,
+                                              void* stream) {
+  int rc = check_desc(d, "shapelet_backward_recompute_input");
+  if (rc) return rc;
+  IGN_REQUIRE(xn && W && g && dxn && ws, "shapelet_backward_recompute_input: null pointer");
+  IGN_REQUIRE(d->dist == IGN_DIST_L1 || st0, "shapelet_backward_recompute_input: dist %d needs the window statistics", d->dist);
+  IGN_REQUIRE(d->dist != IGN_DIST_PEARSON || st1, "shapelet_backward_recompute_input: PEARSON needs st1 (window means)");
+  IGN_REQUIRE(d->pool != IGN_POOL_LTS_MIN || thr, "shapelet_backward_recompute_input: lts_min needs the threshold again");
+  return launch_shapelet_bwd_recompute(*d, xn, st0, st1, W, thr, g, gdmin, dW, dxn, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 int32_t ign_diversity_partials(int32_t K) { return K <= 0 ? 0 : diversity_blocks(K) * diversity_blocks(K); }

@@ -59,10 +59,12 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
 bool shapelet_bwd_coef_offset(const ign_shapelet_desc& d, size_t* off_floats, size_t* total_bytes);
 int launch_shapelet_dx(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1, const float* W,
                        const float* coef, const float* dstore, float* dxn, cudaStream_t st);
-size_t shapelet_bwd_recompute_workspace(const ign_shapelet_desc& d, size_t budget);
+// dx: the layout of the input-gradient walk (dxn != NULL below), which keeps cosine / pearson distances apart
+size_t shapelet_bwd_recompute_workspace(const ign_shapelet_desc& d, size_t budget, bool dx);
+// dW == NULL: weights frozen (needs dxn); dxn == NULL: dW only; dxn != NULL: dxn += the input gradient, chunk by chunk
 int launch_shapelet_bwd_recompute(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1,
                                   const float* W, const float* thr, const float* g, const float* gdmin, float* dW,
-                                  void* ws, size_t ws_bytes, cudaStream_t st);
+                                  float* dxn, void* ws, size_t ws_bytes, cudaStream_t st);
 // engine selection + launch shared by ign_shapelet_forward and the recompute backward (api.cu)
 size_t shapelet_forward_workspace_bytes(const ign_shapelet_desc& d);
 int shapelet_forward_dispatch(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* W,

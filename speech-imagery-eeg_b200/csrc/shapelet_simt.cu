@@ -1703,11 +1703,17 @@ int launch_shapelet_bwd_simt(const ign_shapelet_desc& d, const float* xn, const 
 
 // ---- recompute mode: nothing saved by the forward; bounded workspace, shapelets walked in chunks --------------------
 namespace {
-struct RecomputeLayout { int Kc; size_t bwd_bytes, out_off, fws_off, fws_bytes, total; };
+struct RecomputeLayout { int Kc; size_t bwd_bytes, out_off, fws_off, fws_bytes, dist_off, total; };
 
 size_t align128(size_t v) { return (v + 127) / 128 * 128; }
 
-bool recompute_layout(const ign_shapelet_desc& d, int Kc, RecomputeLayout& r) {
+// The input gradient of cosine / pearson reads the window distances next to the coefficients (launch_shapelet_dx's
+// beta terms), so with dx the chunk's distances get a buffer of their own instead of being converted in place.
+bool dx_keeps_distances(const ign_shapelet_desc& d, bool dx) {
+  return dx && (d.dist == IGN_DIST_COSINE || d.dist == IGN_DIST_PEARSON);
+}
+
+bool recompute_layout(const ign_shapelet_desc& d, int Kc, RecomputeLayout& r, bool dx) {
   ign_shapelet_desc dc = d;
   dc.K = Kc;
   Geo g; BwdPlan bp;
@@ -1717,17 +1723,19 @@ bool recompute_layout(const ign_shapelet_desc& d, int Kc, RecomputeLayout& r) {
   r.out_off = r.bwd_bytes;                                            // p | dmin | argmin of the chunk, [B,Kc,M] each
   r.fws_off = r.out_off + align128((size_t)3 * d.B * Kc * d.M * sizeof(float));
   r.fws_bytes = shapelet_forward_workspace_bytes(dc);
-  r.total = r.fws_off + align128(r.fws_bytes);
+  r.dist_off = r.fws_off + align128(r.fws_bytes);                     // [B,M,Kc,Tw] distances (dx_keeps_distances)
+  r.total = r.dist_off;
+  if (dx_keeps_distances(d, dx)) r.total += align128((size_t)d.B * d.M * Kc * g.Ts * sizeof(float));
   return true;
 }
 
 // largest chunk whose workspace fits `bytes` (a whole number of 8-shapelet blocks unless K itself is smaller), then
 // balanced over the resulting number of chunks
-int recompute_chunk(const ign_shapelet_desc& d, size_t bytes) {
+int recompute_chunk(const ign_shapelet_desc& d, size_t bytes, bool dx) {
   RecomputeLayout r;
   int fit = 0;
   for (int Kc = d.K; Kc >= 1; Kc = (Kc > 8 ? (Kc - 1) / 8 * 8 : Kc - 1)) {
-    if (recompute_layout(d, Kc, r) && r.total <= bytes) { fit = Kc; break; }
+    if (recompute_layout(d, Kc, r, dx) && r.total <= bytes) { fit = Kc; break; }
   }
   if (fit == 0) fit = min(d.K, 8);                                    // budget too small: the minimum chunk
   const int n = ceil_div(d.K, fit);
@@ -1737,42 +1745,54 @@ int recompute_chunk(const ign_shapelet_desc& d, size_t bytes) {
 }
 }  // namespace
 
-size_t shapelet_bwd_recompute_workspace(const ign_shapelet_desc& d, size_t budget) {
+size_t shapelet_bwd_recompute_workspace(const ign_shapelet_desc& d, size_t budget, bool dx) {
   RecomputeLayout r;
-  if (!recompute_layout(d, recompute_chunk(d, budget), r)) return 0;
+  if (!recompute_layout(d, recompute_chunk(d, budget, dx), r, dx)) return 0;
   return r.total;
 }
 
 int launch_shapelet_bwd_recompute(const ign_shapelet_desc& d, const float* xn, const float* st0, const float* st1,
                                   const float* W, const float* thr, const float* gr, const float* gdmin, float* dW,
-                                  void* ws, size_t ws_bytes, cudaStream_t st) {
+                                  float* dxn, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const bool dx = dxn != nullptr;
   if (((uintptr_t)ws & 127) != 0) { set_error("shapelet_backward(recompute): workspace must be 128-byte aligned"); return IGN_ERR_INVALID; }
-  const int Kc = recompute_chunk(d, ws_bytes);
+  const int Kc = recompute_chunk(d, ws_bytes, dx);
   RecomputeLayout r;
-  if (!recompute_layout(d, Kc, r)) { set_error("shapelet_backward(recompute): problem does not fit shared memory (T=%d L=%d)", d.T, d.L); return IGN_ERR_UNSUPPORTED; }
-  if (r.total > ws_bytes) { set_error("shapelet_backward(recompute): workspace %zu < %zu bytes (ign_shapelet_backward_recompute_workspace)", ws_bytes, r.total); return IGN_ERR_INVALID; }
+  if (!recompute_layout(d, Kc, r, dx)) { set_error("shapelet_backward(recompute): problem does not fit shared memory (T=%d L=%d)", d.T, d.L); return IGN_ERR_UNSUPPORTED; }
+  if (r.total > ws_bytes) { set_error("shapelet_backward(recompute): workspace %zu < %zu bytes (%s)", ws_bytes, r.total, dx ? "ign_shapelet_backward_recompute_input_workspace" : "ign_shapelet_backward_recompute_workspace"); return IGN_ERR_INVALID; }
   uint8_t* base8 = reinterpret_cast<uint8_t*>(ws);
   for (int k0 = 0; k0 < d.K; k0 += Kc) {
     ign_shapelet_desc dc = d;
     dc.K = min(Kc, d.K - k0);
     RecomputeLayout rc;
-    if (!recompute_layout(dc, dc.K, rc) || rc.total > ws_bytes) { set_error("shapelet_backward(recompute): internal chunk layout"); return IGN_ERR_INVALID; }
+    if (!recompute_layout(dc, dc.K, rc, dx) || rc.total > ws_bytes) { set_error("shapelet_backward(recompute): internal chunk layout"); return IGN_ERR_INVALID; }
     Geo g; BwdPlan bp;
     base_geo(dc, g); plan_bwd(g, bp);
     const BwdWorkspace wo = bwd_workspace(dc, g, bp);
     float* dbuf = reinterpret_cast<float*>(base8) + wo.coef;            // distances now, coefficients after the pooling pass
+    float* dkeep = dx_keeps_distances(d, dx) ? reinterpret_cast<float*>(base8 + rc.dist_off) : nullptr;
     float* outp = reinterpret_cast<float*>(base8 + rc.out_off);
     const size_t no = (size_t)d.B * dc.K * d.M;
     const size_t wofs = (size_t)k0 * d.M * d.L;
-    // 1. the forward of this chunk again (same kernels, same engine as the real forward): window distances -> dbuf
+    // 1. the forward of this chunk again (same kernels, same engine as the real forward): window distances -> dbuf, or
+    //    -> dkeep when the input gradient reads them after the pooling pass
     int rc1 = shapelet_forward_dispatch(dc, xn, st0, W + wofs, thr ? thr + (size_t)k0 * d.M : nullptr, outp, outp + no,
-                                        reinterpret_cast<int*>(outp + 2 * no), dbuf, base8 + rc.fws_off, rc.fws_bytes, st);
+                                        reinterpret_cast<int*>(outp + 2 * no), dkeep ? dkeep : dbuf, base8 + rc.fws_off,
+                                        rc.fws_bytes, st);
     if (rc1) return rc1;
-    // 2. pooling backward in place, contraction, finalize -> dW[k0 .. k0+Kc); gdmin is read like gr, at the chunk's
-    //    shapelets, and lands on the recomputed argmin of the chunk (the same kernels give the forward's index)
-    rc1 = launch_shapelet_bwd_simt(dc, xn, st0, st1, W + wofs, gr, gdmin, d.K, k0, nullptr, outp + no,
-                                   reinterpret_cast<const int*>(outp + 2 * no), dW + wofs, ws, rc.bwd_bytes, st);
+    // 2. pooling backward (in place, or dkeep -> dbuf), contraction, finalize -> dW[k0 .. k0+Kc) (dW == NULL: the
+    //    pooling backward alone); gdmin is read like gr, at the chunk's shapelets, and lands on the recomputed argmin of
+    //    the chunk (the same kernels give the forward's index)
+    rc1 = launch_shapelet_bwd_simt(dc, xn, st0, st1, W + wofs, gr, gdmin, d.K, k0, dkeep, outp + no,
+                                   reinterpret_cast<const int*>(outp + 2 * no), dW ? dW + wofs : nullptr, ws,
+                                   rc.bwd_bytes, st);
     if (rc1) return rc1;
+    // 3. dxn += this chunk's shapelets' share.  Every dxn row belongs to one CTA, which adds the shapelets in k order:
+    //    chunk after chunk on one stream, the sum over k runs in the stored mode's order.
+    if (dx) {
+      rc1 = launch_shapelet_dx(dc, xn, st0, st1, W + wofs, dbuf, dkeep, dxn, st);
+      if (rc1) return rc1;
+    }
   }
   return IGN_OK;
 }

@@ -55,6 +55,8 @@ _SIGNATURES = {
     "ign_shapelet_backward": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 11 + [c_size_t, _P]),
     "ign_shapelet_backward_dmin": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 12 + [c_size_t, _P]),
     "ign_shapelet_backward_input": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 7 + [c_size_t, _P]),
+    "ign_shapelet_backward_recompute_input_workspace": (c_size_t, [POINTER(ShapeletDesc), c_size_t]),
+    "ign_shapelet_backward_recompute_input": (c_int32, [POINTER(ShapeletDesc)] + [_P] * 10 + [c_size_t, _P]),
     "ign_diversity_partials": (c_int32, [c_int32]),
     "ign_diversity_forward": (c_int32, [_P, _P, _P, c_int32, c_int32, c_int32, _P]),
     "ign_diversity_backward": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, _P]),

@@ -216,7 +216,8 @@ class _InstanceNorm(torch.autograd.Function):
 def instance_norm(x: torch.Tensor) -> SeriesPack:
     """x [B,T,M] -> SeriesPack(xn [B,M,Tp]).  Shapelet.py:186-187.  In the reference's training loop the raw batch never
     requires grad (experiment_classification.py:315); when it does (saliency), the pack carries an autograd variable
-    and the shapelet transform returns dLoss/dxn through ign_shapelet_backward_input."""
+    and the shapelet transform returns dLoss/dxn through ign_shapelet_backward_input (stored-distance groups) or
+    ign_shapelet_backward_recompute_input (recompute groups)."""
     _require_cuda(x, "x")
     if x.dim() != 3:
         raise RuntimeError("instance_norm expects [B,T,M], got %s" % (tuple(x.shape),))
@@ -305,6 +306,8 @@ def _backward_group(rec: _Group, pack: SeriesPack, saved, g_p, g_dmin, need_dx):
     st0, st1 = pack.window_stats(rec.dist, desc.L, desc.stride)
     if rec.stored:
         nbytes = C.lib.ign_shapelet_backward_workspace(byref(desc))
+    elif need_dx:   # recompute mode with dx: one call per group, as no chunk's coefficients outlive the chunk
+        nbytes = C.lib.ign_shapelet_backward_recompute_input_workspace(byref(desc), STORE_BUDGET_BYTES)
     else:       # recompute mode: the library walks the shapelets in chunks inside this bounded workspace
         nbytes = C.lib.ign_shapelet_backward_recompute_workspace(byref(desc), STORE_BUDGET_BYTES)
     dW = torch.empty_like(Wc) if need_w else None      # None: the library only prepares the coefficients for dxn
@@ -316,6 +319,11 @@ def _backward_group(rec: _Group, pack: SeriesPack, saved, g_p, g_dmin, need_dx):
         head = (byref(desc), _ptr(pack.xn), _ptr(st0), _ptr(st1), _ptr(Wc), _ptr(thr), _ptr(g))
         tail = (_ptr(dstore), _ptr(out[1]), _ptr(idx), _ptr(dW), _ptr(ws), int(nbytes), _stream())
         with torch.cuda.device(g.device):
+            if dxn is not None and not rec.stored:
+                C.check(STATS.call(tag, 3 if need_w else 2, lambda: C.lib.ign_shapelet_backward_recompute_input(
+                    *head, _ptr(gd), _ptr(dW), _ptr(dxn), _ptr(ws), int(nbytes), _stream())),
+                    "ign_shapelet_backward_recompute_input")
+                return
             if gd is None:
                 C.check(STATS.call(tag, 2 if need_w else 1, lambda: C.lib.ign_shapelet_backward(*head, *tail)),
                         "ign_shapelet_backward")
@@ -361,10 +369,6 @@ class _SbmTransform(torch.autograd.Function):
             need = bool(track and (nW or nT or need_dx))
             rec, o, saved = _forward_group(pack, W, thr, stride, eps, dist, pool, precision, need)
             rec.needs = (need, nW, nT)
-            if need_dx and need and not rec.stored:
-                raise NotImplementedError("ign_b200: the input gradient needs the stored-distance backward; raise "
-                                          "IGN_BWD_STORE_BUDGET_GB (this group would keep %d bytes)" % (
-                                              2 * int(C.lib.ign_shapelet_dstore_bytes(byref(rec.desc)))))
             recs.append(rec); outs.extend(o); saved_all.extend(saved)
         ctx.set_materialize_grads(False)
         ctx.recs, ctx.pack, ctx.need_dx = recs, pack, need_dx
